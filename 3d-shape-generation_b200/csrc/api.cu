@@ -150,19 +150,10 @@ struct pcd_denoiser {
     int T = 256;       // dim == time_dim of the checkpoint (networks.py:737-744): width of the time MLP and of enc1.conv1's temb columns
     int f16 = 0;       // 16-bit format of weights/activations: 0 = bf16, 1 = fp16
     int planes = 1;    // 2 = every 16-bit tensor carries a hi and a lo plane (split operands, 3 MMAs per k-step)
-    bool two_pass[L_COUNT] = {};      // planes == 2 only: split layers that skip the (activation lo) x (weight hi) pass
-    bool single_pass[L_COUNT] = {};   // planes == 2 only: layers that still run ONE pass on the hi planes (PCD_PRECISION_F16MIX)
+    bool single_pass[L_COUNT] = {};   // f16mix only: layers that still run ONE pass on the hi planes (kMixSinglePass)
     bool c8[L_COUNT] = {};            // f16mix only: split layers whose two correction terms run as ONE fp8 (e5m2) pass (gemm_tc.cu NP == 4);
                                       // their weights carry a third plane (the e5m2 byte plane) and their inputs' second plane is a byte plane
-    int cluster = 2;   // CTA-pair clusters (PCD_CLUSTER=1 disables)
-    int two_sm = 1;    // 1: pairs run the pair MMA (cta_group::2) on layers with K >= 1024, TMA multicast + per-CTA MMAs elsewhere
-                       // (measured: +5-6 % on K >= 1024, -15 % on K <= 512 where per-tile hand-shakes dominate); PCD_2SM=0 never, 2 always
     bool taps = false;
-    int chain = -1;        // fuse the narrow layer chains (enc1+enc2, dec1+output) into one kernel each (chain_tc.cu): -1 = for plans of at most
-                           // 4 row tiles per SM (batch <= 37 at 2048 points), where launch / drain latency dominates; PCD_CHAIN=0 never, 1 always
-    int epi_warps = 8;     // store epilogue: two warps per TMEM lane quarter (PCD_EPI_WARPS=4: one, the round-1 form)
-    int tile_order = -1;   // PCD_TILE_ORDER: -1 = per layer (n fastest where two planes make the row-block working set outgrow L2), 0 / 1 = force
-    int x3_wide = 1, x3_wide_min_k = 512;   // split-precision layers with cout >= 256 and K >= min_k: 256-column tiles on the pair MMA
     // GEMM layers in execution order (index constants below)
     std::vector<DevLayer> L;
     // small fp32 pieces
@@ -213,6 +204,14 @@ static const int kConsumers[L_COUNT][2] = {
     /*E4C3*/ {L_G0, L_D4C1}, /*G0*/ {L_G3, -1}, /*G3*/ {-1, -1}, /*D4C1*/ {L_D4C2, -1}, /*D4C2*/ {L_D4C3, -1}, /*D4C3*/ {L_D3C1, -1},
     /*D3C1*/ {L_D3C2, -1}, /*D3C2*/ {L_D3C3, -1}, /*D3C3*/ {L_D2C1, -1}, /*D2C1*/ {L_D2C2, -1}, /*D2C2*/ {L_D2C3, -1},
     /*D2C3*/ {L_D1C1, -1}, /*D1C1*/ {L_D1C2, -1}, /*D1C2*/ {L_D1C3, -1}, /*D1C3*/ {L_O0, -1}, /*O0*/ {-1, -1}};
+
+// f16mix: global_feat.0 / global_feat.3 hold 67 % of the FLOPs and each contributes only ~3-4.5e-4 relative error when run as ONE
+// fp16 pass (measured per layer against the fp32 oracle); dec4.conv1 (6.7 % of the FLOPs, ~3.6e-4) as well: eps error 4.7e-4 ->
+// ~6e-4, step time -8 %.  Everything else stays split (3 passes).
+static const int kMixSinglePass[] = {L_G0, L_G3, L_D4C1};
+// f16mix: the tensor-bound split layers (K >= 512: enc4.*, dec4.conv2/3, dec3.*; 46 % of the split-mode step) run their two correction
+// terms as one fp8 pass: 2 pass-equivalents instead of 3.  Every one has cout >= 256: the fp8 form needs 256-column pair-MMA tiles.
+static const int kMixC8[] = {L_E4C1, L_E4C2, L_E4C3, L_D4C2, L_D4C3, L_D3C1, L_D3C2, L_D3C3};
 
 // pass structure of a layer in a plan: 1 = one pass on the hi planes, 3 = split (hi*hi + hi*lo + lo*hi), 4 = hi*hi + one fp8 pass
 static int layer_np(const pcd_denoiser* h, int layer, bool plan_c8) {
@@ -283,66 +282,11 @@ extern "C" int pcd_denoiser_create(const pcd_named_tensor* tensors, int32_t n_te
     h->f16 = (precision == PCD_PRECISION_F16 || precision == PCD_PRECISION_F16MIX) ? 1 : 0;
     h->planes = (precision == PCD_PRECISION_BF16X3 || precision == PCD_PRECISION_F16MIX) ? 2 : 1;
     if (precision == PCD_PRECISION_F16MIX) {
-        // global_feat.0 / global_feat.3 hold 67 % of the FLOPs and each contributes only ~3-4.5e-4 relative error when
-        // run as ONE fp16 pass (measured per layer against the fp32 oracle); everything else stays split (3 passes).
-        h->single_pass[L_G3] = true;
-        h->single_pass[L_G0] = true;
-        // dec4.conv1 (6.7 % of the FLOPs, ~3.6e-4) as well unless PCD_MIX2=1: eps error 4.7e-4 -> ~6e-4, step time -8 %
-        if (std::getenv("PCD_MIX2") == nullptr) h->single_pass[L_D4C1] = true;
-        // experiments: PCD_MIX_EXTRA=d4c2,d4c3,... adds layers to the single-pass set
-        if (const char* extra = std::getenv("PCD_MIX_EXTRA")) {
-            static const struct { const char* n; int id; } names[] = {
-                {"e1c2", L_E1C2}, {"e1c3", L_E1C3}, {"e2c1", L_E2C1}, {"e2c2", L_E2C2}, {"e2c3", L_E2C3}, {"e3c1", L_E3C1}, {"e3c2", L_E3C2},
-                {"e3c3", L_E3C3}, {"e4c1", L_E4C1}, {"e4c2", L_E4C2}, {"e4c3", L_E4C3}, {"d4c2", L_D4C2}, {"d4c3", L_D4C3}, {"d3c1", L_D3C1},
-                {"d3c2", L_D3C2}, {"d3c3", L_D3C3}, {"d2c1", L_D2C1}, {"d2c2", L_D2C2}, {"d2c3", L_D2C3}, {"d1c1", L_D1C1}, {"d1c2", L_D1C2},
-                {"d1c3", L_D1C3}, {"o0", L_O0}};
-            const std::string ex = std::string(",") + extra + ",";
-            for (const auto& nm : names)
-                if (ex.find(std::string(",") + nm.n + ",") != std::string::npos) h->single_pass[nm.id] = true;
-        }
-        // the tensor-bound split layers (K >= 512: enc4.*, dec4.conv2/3, dec3.*; 46 % of the split-mode step) run their two
-        // correction terms as one fp8 pass: 2 pass-equivalents instead of 3.  PCD_MIX_C8=none disables, =e3c3,... replaces the set
-        {
-            static const struct { const char* n; int id; } names[] = {
-                {"e2c3", L_E2C3}, {"e3c1", L_E3C1}, {"e3c2", L_E3C2}, {"e3c3", L_E3C3}, {"e4c1", L_E4C1}, {"e4c2", L_E4C2}, {"e4c3", L_E4C3},
-                {"d4c2", L_D4C2}, {"d4c3", L_D4C3}, {"d3c1", L_D3C1}, {"d3c2", L_D3C2}, {"d3c3", L_D3C3}, {"d2c1", L_D2C1}, {"d2c2", L_D2C2},
-                {"d2c3", L_D2C3}};
-            const char* env = std::getenv("PCD_MIX_C8");
-            const std::string ex = std::string(",") + (env ? env : "e4c1,e4c2,e4c3,d4c2,d4c3,d3c1,d3c2,d3c3") + ",";
-            for (const auto& nm : names)
-                if (ex.find(std::string(",") + nm.n + ",") != std::string::npos) h->c8[nm.id] = true;
-        }
-        // experiments: PCD_MIX_NP2=d4c2,d4c3,... runs split layers as two passes (no activation-lo pass)
-        if (const char* extra = std::getenv("PCD_MIX_NP2")) {
-            static const struct { const char* n; int id; } names[] = {
-                {"e1c2", L_E1C2}, {"e1c3", L_E1C3}, {"e2c1", L_E2C1}, {"e2c2", L_E2C2}, {"e2c3", L_E2C3}, {"e3c1", L_E3C1}, {"e3c2", L_E3C2},
-                {"e3c3", L_E3C3}, {"e4c1", L_E4C1}, {"e4c2", L_E4C2}, {"e4c3", L_E4C3}, {"d4c2", L_D4C2}, {"d4c3", L_D4C3}, {"d3c1", L_D3C1},
-                {"d3c2", L_D3C2}, {"d3c3", L_D3C3}, {"d2c1", L_D2C1}, {"d2c2", L_D2C2}, {"d2c3", L_D2C3}, {"d1c1", L_D1C1}, {"d1c2", L_D1C2},
-                {"d1c3", L_D1C3}, {"o0", L_O0}};
-            const std::string ex = std::string(",") + extra + ",";
-            for (const auto& nm : names)
-                if (ex.find(std::string(",") + nm.n + ",") != std::string::npos) h->two_pass[nm.id] = true;
-        }
+        for (int l : kMixSinglePass) h->single_pass[l] = true;
+        for (int l : kMixC8) h->c8[l] = true;
     }
     h->taps = std::getenv("PCD_TAPS") != nullptr;
-    if (const char* c = std::getenv("PCD_CLUSTER")) h->cluster = std::atoi(c) == 2 ? 2 : 1;
-    if (const char* c = std::getenv("PCD_2SM")) h->two_sm = std::atoi(c);
-    if (const char* c = std::getenv("PCD_X3_WIDE")) h->x3_wide = std::atoi(c) != 0;
-    if (const char* c = std::getenv("PCD_X3_WIDE_MIN_K")) h->x3_wide_min_k = std::atoi(c);
-    if (const char* c = std::getenv("PCD_TILE_ORDER")) h->tile_order = std::atoi(c);
-    if (const char* c = std::getenv("PCD_EPI_WARPS")) h->epi_warps = std::atoi(c) == 4 ? 4 : 8;
-    if (const char* c = std::getenv("PCD_CHAIN")) h->chain = std::atoi(c);
     h->L.resize(L_COUNT);
-    {
-        static const int couts[L_COUNT] = {64, 128, 128, 128, 256, 256, 256, 512, 512, 512, 1024, 2048, 4096, 1024, 1024, 512, 512, 512, 256,
-                                           256, 256, 128, 128, 128, 64, 64};
-        for (int l = 0; l < L_COUNT; ++l) {
-            if (h->single_pass[l] || h->two_pass[l] || couts[l] < 256) h->c8[l] = false;   // the fp8 form needs 256-column pair-MMA tiles
-        }
-        for (int l = 0; l < L_COUNT; ++l)
-            REQ(out_format(h.get(), l, true) > 0, std::string("PCD_MIX_C8: the consumers of ") + std::to_string(l) +
-                " disagree on the format of its second plane (16-bit residual vs e5m2 byte plane)");
-    }
 
 #define FOLD(dst, conv, bn, co, ci) \
     HostMat dst;                    \
@@ -530,7 +474,6 @@ static int add_gemm(pcd_denoiser* h, Plan* pl, int layer, const void* a0, int k0
     const long long Mrows = pl->M * PLn;        // hi plane rows [0, M), lo plane rows [M, 2M)
     op.np = layer_np(h, layer, pl->c8);   // a single-pass layer reads (and writes) hi planes only
     p.f16 = h->f16;
-    p.np2 = (op.np == 3 && h->two_pass[layer] && epi != EPI_MAXPOOL) ? 1 : 0;
     // a STORE layer writes the second plane its consumers read: nothing when every consumer is single-pass (global_feat.0 ->
     // global_feat.3, and enc4.conv3 (x4) -> global_feat.0 + dec4.conv1 in f16mix), the 16-bit residual for split consumers, the
     // e5m2 byte plane for fp8-corrected consumers
@@ -541,12 +484,11 @@ static int add_gemm(pcd_denoiser* h, Plan* pl, int layer, const void* a0, int k0
     p.kb0 = k0 / 64; p.kb1 = k1 / 64;
     p.bias = bias; p.bias_sample_stride = sample_bias_stride; p.rows_per_sample = pl->Npad; p.relu = 1;
     p.gmax = pl->gmax; p.ld_g = 4096; p.n_valid = pl->N; p.num_samples = pl->B; p.call = pl->call;
-    if (const char* d = std::getenv("PCD_DBG")) p.dbg = std::atoi(d);
     if (epi == EPI_MAXPOOL) {
         // weights take the A role (128 channels per tile), points the B role
         op.bn = (op.np == 1 && pl->M % 256 == 0) ? 256 : 128;
         p.num_m_blocks = L.cout / 128; p.num_n_blocks = static_cast<int>(pl->M / op.bn);
-        op.cl = (h->cluster == 2 && p.num_m_blocks % 2 == 0) ? 2 : 1;
+        op.cl = p.num_m_blocks % 2 == 0 ? 2 : 1;
         p.a_plane_rows = PLn == 2 ? L.cout : 0; p.b_plane_rows = PLn == 2 ? static_cast<int>(pl->M) : 0; p.out_plane_rows = 0;
         if (make_tmap(&op.a0, L.w16, static_cast<long long>(L.cout) * PLn, L.k, L.k, 128)) return 1;
         op.a1 = op.a0;
@@ -554,10 +496,10 @@ static int add_gemm(pcd_denoiser* h, Plan* pl, int layer, const void* a0, int k0
         op.o = op.a0;
     } else {
         p.num_m_blocks = static_cast<int>(pl->M / 128);
-        op.cl = (h->cluster == 2 && p.num_m_blocks % 2 == 0) ? 2 : 1;
+        op.cl = p.num_m_blocks % 2 == 0 ? 2 : 1;
         // split precision (3 passes, 2 planes): 128-column tiles, or 256-column tiles on the pair MMA where each CTA stages only half
-        // of the B tile (halves the L2->SM bytes per FLOP; PCD_X3_WIDE=0 disables)
-        const bool wide3 = op.np == 4 || (op.np == 3 && op.cl == 2 && h->two_sm != 0 && L.cout >= 256 && h->x3_wide && k0 + k1 >= h->x3_wide_min_k);
+        // of the B tile (halves the L2->SM bytes per FLOP)
+        const bool wide3 = op.np == 4 || (op.np == 3 && op.cl == 2 && L.cout >= 256 && k0 + k1 >= 512);
         op.bn = op.np >= 3 ? (wide3 ? 256 : (L.cout >= 128 ? 128 : L.cout)) : (L.cout >= 256 ? 256 : L.cout);
         p.num_n_blocks = L.cout / op.bn;
         p.out = static_cast<__nv_bfloat16*>(dst); p.ldo = L.cout;
@@ -568,11 +510,9 @@ static int add_gemm(pcd_denoiser* h, Plan* pl, int layer, const void* a0, int k0
         if (k1 > 0) { if (make_tmap(&op.a1, a1, Mrows, k1, k1, 128)) return 1; }
         else op.a1 = op.a0;
         if (make_tmap(&op.b, L.w16, static_cast<long long>(L.cout) * L.wplanes, L.k, L.k, op.bn / op.cl)) return 1;
-        p.epi_warps = (epi == EPI_STORE && L.cout >= 64) ? h->epi_warps : 4;
-        if (epi == EPI_STORE) {
-            if (p.epi_warps == 8) { if (make_tmap_out32(&op.o, dst, Mrows, L.cout, L.cout)) return 1; }
-            else if (make_tmap(&op.o, dst, Mrows, L.cout, L.cout, 32)) return 1;
-        }
+        // STORE layers: two epilogue warps per TMEM lane quarter (the 32 x 32 store map)
+        p.epi_warps = epi == EPI_STORE ? 8 : 4;
+        if (epi == EPI_STORE) { if (make_tmap_out32(&op.o, dst, Mrows, L.cout, L.cout)) return 1; }
         else op.o = op.a0;
     }
     if (epi != EPI_MAXPOOL) {
@@ -580,9 +520,11 @@ static int add_gemm(pcd_denoiser* h, Plan* pl, int layer, const void* a0, int k0
         // (profiles/tile_order_ab_r2.jsonl): n fastest wins where that set is >= 38 MB and the layer has 2..4 weight tiles
         // (dec4.conv2 in f16mix: 3.68 -> 3.10 ms); with 8 weight tiles (global_feat.0) the default order stays ahead by 1-3 %.
         const double live_mb = static_cast<double>(h->num_sms) * 128.0 * (k0 + k1) * 2.0 * (op.np >= 3 ? 2 : 1) / (1 << 20);
-        p.tile_order = h->tile_order >= 0 ? h->tile_order : ((p.num_n_blocks >= 2 && p.num_n_blocks <= 4 && live_mb > 30.0) ? 1 : 0);
+        p.tile_order = (p.num_n_blocks >= 2 && p.num_n_blocks <= 4 && live_mb > 30.0) ? 1 : 0;
     }
-    op.two_sm = (op.cl == 2 && (h->two_sm == 2 || (h->two_sm == 1 && k0 + k1 >= 1024))) ? 1 : 0;
+    // pairs run the pair MMA (cta_group::2) on layers with K >= 1024, TMA multicast + per-CTA MMAs elsewhere (measured: +5-6 % on
+    // K >= 1024, -15 % on K <= 512 where per-tile hand-shakes dominate)
+    op.two_sm = (op.cl == 2 && k0 + k1 >= 1024) ? 1 : 0;
     if (op.np >= 3 && op.bn == 256) op.two_sm = 1;
     if (np3_one_plane && op.bn != 256) op.out_planes = 2;
     if (layer == L_E3C3) pl->fmtX3 = op.out_planes;
@@ -627,15 +569,17 @@ static int add_chain(pcd_denoiser* h, Plan* pl, int chain_id, const std::vector<
     return 0;
 }
 
-// the chains run every layer as plain one-pass or three-pass layers with 16-bit residual planes: no experiments inside them
+// the chains run every layer as plain one-pass or three-pass layers with 16-bit residual planes: no single-pass or fp8-corrected
+// f16mix layer inside them.  They are used for plans of at most 4 row tiles per SM (batch <= 37 at 2048 points), where launch /
+// drain latency dominates.
 static bool chain_ok(const pcd_denoiser* h, const Plan* pl, std::initializer_list<int> layers, int last_out_layer) {
-    if (h->chain == 0 || h->precision == PCD_PRECISION_FP32) return false;
+    if (h->precision == PCD_PRECISION_FP32) return false;
     // Measured (profiles/chain_fused_ab_r2.jsonl, profiles/chain_fused_timing_r2.jsonl): batch 4 gains 8-9 % (11 launches become 2), batch 64
     // is neutral, batch 512 LOSES (f16mix: 0.97 -> 1.20 ms for enc1+enc2, bf16: 0.51 -> 0.93): inside a chain a tile's epilogue and its next
     // layer's MMAs are serial, while the per-layer kernels overlap them across tiles and already run at 73-89 % of the HBM rate.
-    if (h->chain < 0 && pl->M / 128 > 4LL * h->num_sms) return false;
+    if (pl->M / 128 > 4LL * h->num_sms) return false;
     for (int l : layers)
-        if (h->single_pass[l] || h->two_pass[l] || h->c8[l]) return false;
+        if (h->single_pass[l] || h->c8[l]) return false;
     if (pl->planes == 2 && last_out_layer >= 0 && out_format(h, last_out_layer, pl->c8) != 2) return false;
     return true;
 }
@@ -656,7 +600,7 @@ static int build_plan(pcd_denoiser* h, int B, int N, Plan** out) {
     pl->elt = h->precision == PCD_PRECISION_FP32 ? 4 : 2;
     pl->planes = h->planes;
     // the fp8-corrected form exists on the pair MMA only: a plan whose row blocks do not pair up runs those layers as plain split layers
-    pl->c8 = h->planes == 2 && h->cluster == 2 && h->two_sm != 0 && (pl->M / 128) % 2 == 0;
+    pl->c8 = h->planes == 2 && (pl->M / 128) % 2 == 0;
     const size_t e = static_cast<size_t>(pl->elt) * pl->planes, M = static_cast<size_t>(pl->M);
     if (plan_alloc(pl.get(), &pl->X1, M * 128 * e) || plan_alloc(pl.get(), &pl->X2, M * 256 * e) ||
         plan_alloc(pl.get(), &pl->X3, M * 512 * e) || plan_alloc(pl.get(), &pl->X4, M * 1024 * e) ||
@@ -779,8 +723,7 @@ static int run_step(pcd_denoiser* h, Plan* pl, cudaStream_t s, bool advance, std
                 p.bias = h->bg; p.bias_sample_stride = 0; p.rows_per_sample = 1 << 30; p.relu = 0;
                 p.partial = pl->dpartial; p.splits = pl->dsplits;
                 // batches of at most 8: one CTA per (32 columns, k split) with the tiled kernel's accumulation order (bit-identical)
-                const bool skinny = std::getenv("PCD_SKINNY") == nullptr || std::atoi(std::getenv("PCD_SKINNY")) != 0;
-                if (skinny && skinny_splitk_ok(p)) { CU(launch_skinny_splitk(p, s)); }
+                if (skinny_splitk_ok(p)) { CU(launch_skinny_splitk(p, s)); }
                 else { CU(launch_gemm_simt(EPI_STORE, p, s)); }
                 ++launched;
                 if (pl->dsplits > 1) { CU(launch_splitk_reduce(pl->dpartial, pl->dsplits, h->bg, pl->biasd4, pl->B, 1024, 0, s)); ++launched; }
@@ -1066,16 +1009,13 @@ extern "C" int pcd_linear_bf16(const void* A0, int32_t K0, const void* A1, int32
     if (make_tmap(&a0, A0, M, K0, K0, 128)) return 1;
     if (K1 > 0) { REQ(A1 != nullptr, "A1 is null but K1 > 0"); if (make_tmap(&a1, A1, M, K1, K1, 128)) return 1; }
     else a1 = a0;
-    const char* cenv = std::getenv("PCD_CLUSTER");
-    const int cl = ((cenv == nullptr || std::atoi(cenv) == 2) && (M / 128) % 2 == 0) ? 2 : 1;
+    const int cl = (M / 128) % 2 == 0 ? 2 : 1;
     if (make_tmap(&b, W, Cout, K0 + K1, K0 + K1, bn / cl)) return 1;
     TcGemmParams p{};
     p.num_m_blocks = M / 128; p.num_n_blocks = Cout / bn; p.kb0 = K0 / 64; p.kb1 = K1 / 64;
     p.out = static_cast<__nv_bfloat16*>(out); p.ldo = Cout; p.bias = bias; p.bias_sample_stride = 0;
     p.rows_per_sample = 1 << 30; p.relu = relu;
-    const char* tenv = std::getenv("PCD_2SM");
-    const int tmode = tenv ? std::atoi(tenv) : 1;
-    const int two_sm = (cl == 2 && (tmode == 2 || (tmode == 1 && K0 + K1 >= 1024))) ? 1 : 0;
+    const int two_sm = (cl == 2 && K0 + K1 >= 1024) ? 1 : 0;
     LAUNCH(launch_gemm_tc(bn, EPI_STORE, 1, 1, cl, two_sm, a0, a1, b, o, p, sms, static_cast<cudaStream_t>(stream)));
     return 0;
 }

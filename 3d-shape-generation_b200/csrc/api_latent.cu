@@ -54,10 +54,9 @@ struct pcd_latent {
     Lin dec4c, dec3c, dec2c, dec1c;   // decK with refineK composed into its skip columns (persistent-kernel path)
     float *tw0 = nullptr, *tw2 = nullptr;   // time MLP weights [out][in]
     // tile-major, pre-swizzled copies streamed by the persistent kernel (latent_mk.cu: tile_weights_kernel)
-    float *t_tw0 = nullptr, *t_tw2 = nullptr, *t_enc1z = nullptr, *t_enc1t = nullptr, *t_enc2 = nullptr, *t_enc3 = nullptr,
-          *t_enc4 = nullptr, *t_gf0 = nullptr, *t_gf3 = nullptr, *t_dec4 = nullptr, *t_dec3 = nullptr, *t_dec2 = nullptr,
-          *t_dec1 = nullptr, *t_out0 = nullptr, *t_out2 = nullptr, *t_vd0 = nullptr, *t_vd2 = nullptr, *t_vd4 = nullptr,
-          *t_vout = nullptr;
+    float *t_tw0 = nullptr, *t_tw2 = nullptr, *t_enc1t = nullptr, *t_enc3 = nullptr, *t_enc4 = nullptr, *t_gf0 = nullptr,
+          *t_gf3 = nullptr, *t_dec4 = nullptr, *t_dec3 = nullptr, *t_dec2 = nullptr, *t_vd0 = nullptr, *t_vd2 = nullptr,
+          *t_vd4 = nullptr, *t_vout = nullptr;
     int mk_grid = 0;                  // CTAs of the persistent kernel (0: unavailable)
     Lin vd0, vd2, vd4, vout;   // SimplePointNetVAE decoder
     float *out0T = nullptr, *out2T = nullptr;   // output.0 / output.2 weights transposed [in][out] for the row-per-CTA tail phase
@@ -68,7 +67,6 @@ struct pcd_latent {
     // FoldingDecoder (PointNetVAE.decode, networks.py:1449-1509), composed at load time (see folding.cu)
     struct Fold { Lin wz, wab, wbc; float *wg = nullptr, *wc2 = nullptr, *bc2 = nullptr; int kin = 0;
                   void* wab16 = nullptr; /* W_ab as fp16 hi / lo planes [2 * 512][512] for the tcgen05 path */ } fold[2];
-    bool fold_tc = false;      // the 512 x 512 GEMMs of the folds run on the split-precision tcgen05 kernel (sm_100; PCD_FOLD_SIMT=1 disables)
     Lin upsample;
     float* grid = nullptr;     // [1024][2]
     bool has_folding = false;
@@ -165,10 +163,11 @@ static int load_folding(pcd_latent* h, const TensorTable& tt, int num_points) {
         }
     }
     {
+        // the 512 x 512 GEMMs of the folds run on the split-precision tcgen05 kernel
         cudaDeviceProp prop;
         CU(cudaGetDeviceProperties(&prop, h->device));
-        h->fold_tc = prop.major == 10 && std::getenv("PCD_FOLD_SIMT") == nullptr;
-        if (h->fold_tc) CU(configure_gemm_tc());
+        REQ(prop.major == 10, "FoldingDecoder: the tcgen05 path requires an sm_100-class GPU (B200)");
+        CU(configure_gemm_tc());
     }
     const float *wu, *bu, *grid;
     if (!fetch(tt, "vae.decoder.upsample.weight", 1024LL * num_points, &wu, &err) ||
@@ -299,13 +298,10 @@ extern "C" int pcd_latent_create(const pcd_named_tensor* tensors, int32_t n_tens
             if (up(p, wt.data(), wt.size(), &p->dec1cT)) return 1;
         }
         if (tile_w(p, p->tw0, 256, 0, 256, 256, &p->t_tw0) || tile_w(p, p->tw2, 256, 0, 256, 256, &p->t_tw2) ||
-            tile_w(p, p->enc1.w, 512, 0, 128, 256, &p->t_enc1z) || tile_w(p, p->enc1.w, 512, 256, 128, 256, &p->t_enc1t) ||
-            tile_w(p, p->enc2.w, 128, 0, 256, 128, &p->t_enc2) || tile_w(p, p->enc3.w, 256, 0, 512, 256, &p->t_enc3) ||
+            tile_w(p, p->enc1.w, 512, 256, 128, 256, &p->t_enc1t) || tile_w(p, p->enc3.w, 256, 0, 512, 256, &p->t_enc3) ||
             tile_w(p, p->enc4.w, 512, 0, 1024, 512, &p->t_enc4) || tile_w(p, p->gf0.w, 1024, 0, 2048, 1024, &p->t_gf0) ||
             tile_w(p, p->gf3.w, 2048, 0, 4096, 2048, &p->t_gf3) || tile_w(p, p->dec4c.w, 5120, 0, 1024, 5120, &p->t_dec4) ||
-            tile_w(p, p->dec3c.w, 1536, 0, 512, 1536, &p->t_dec3) || tile_w(p, p->dec2c.w, 768, 0, 256, 768, &p->t_dec2) ||
-            tile_w(p, p->dec1c.w, 384, 0, 128, 384, &p->t_dec1) || tile_w(p, p->out0.w, 128, 0, 128, 128, &p->t_out0) ||
-            tile_w(p, p->out2.w, 128, 0, 256, 128, &p->t_out2))
+            tile_w(p, p->dec3c.w, 1536, 0, 512, 1536, &p->t_dec3) || tile_w(p, p->dec2c.w, 768, 0, 256, 768, &p->t_dec2))
             return 1;
     }
     if (p->has_vae && (num_points * 3) % 64 == 0) {
@@ -485,21 +481,13 @@ static int mk_prepare(pcd_latent* h, LatentPlan* pl, int R) {
     P.ops[n++] = lt_gemm(pl->th, 256, nullptr, 0, h->t_tw2, 256, 1, LT_BIAS, pl->tembR, h->b2, 1);
     P.ops[n++] = lt_gemm(pl->tembR, 256, nullptr, 0, h->t_enc1t, 128, 1, LT_BIAS, pl->bias1, h->enc1.b, 1);
     P.n_pre = n;
-    // every reverse step (A0 == nullptr: the caller's z).  enc1 + enc2 as ONE rows-per-CTA phase (latent_mk.cu, head_phase), for every
-    // batch size so that a row's arithmetic does not depend on the batch it is in (PCD_LT_NO_HEAD=1: four tile-job / GroupNorm phases)
-    const bool head = std::getenv("PCD_LT_NO_HEAD") == nullptr;
-    if (head) {
+    // every reverse step (the head reads the caller's z).  enc1 + enc2 as ONE rows-per-CTA phase (latent_mk.cu, head_phase), for every
+    // batch size so that a row's arithmetic does not depend on the batch it is in
+    {
         LtOp hd = lt_norm(nullptr, 0, pl->bias1, h->enc1.gamma, h->enc1.beta, 1, 128, pl->z1);
         hd.kind = LT_HEAD; hd.bias_mode = 1; hd.bias_ld = 128;
         hd.W2 = h->enc1zT; hd.W3 = h->enc2T; hd.b3 = h->enc2.b; hd.gamma2 = h->enc2.gamma; hd.beta2 = h->enc2.beta; hd.out2 = pl->z2;
         P.ops[n++] = hd;
-    } else {
-        const int ks = pick_ks(128, 256);
-        P.ops[n++] = lt_gemm(nullptr, 256, nullptr, 0, h->t_enc1z, 128, ks, LT_PARTIAL, pl->partial, nullptr, 0);
-        LtOp nm = lt_norm(pl->partial, ks, pl->bias1, h->enc1.gamma, h->enc1.beta, 1, 128, pl->z1);
-        nm.bias_mode = 1; nm.bias_ld = 128;
-        P.ops[n++] = nm;
-        lt_layer(&P, &n, h->enc2, h->t_enc2, pl->z1, 128, nullptr, 0, pl->partial, pl->z2, 1);
     }
     lt_layer(&P, &n, h->enc3, h->t_enc3, pl->z2, 256, nullptr, 0, pl->partial, pl->z3, 1);
     lt_layer(&P, &n, h->enc4, h->t_enc4, pl->z3, 512, nullptr, 0, pl->partial, pl->z4, 1);
@@ -508,29 +496,15 @@ static int mk_prepare(pcd_latent* h, LatentPlan* pl, int R) {
     lt_layer(&P, &n, h->dec4c, h->t_dec4, pl->g1, 4096, pl->z4, 1024, pl->partial, pl->d4, 1);   // cat([global, refine4(z4)]) :1080
     lt_layer(&P, &n, h->dec3c, h->t_dec3, pl->d4, 1024, pl->z3, 512, pl->partial, pl->d3, 1);
     lt_layer(&P, &n, h->dec2c, h->t_dec2, pl->d3, 512, pl->z2, 256, pl->partial, pl->d2, 1);
-    // dec1's GroupNorm, output.0, output.2 and the update as ONE rows-per-CTA phase (latent_mk.cu, tail_phase), for every batch size
-    // so that a row's arithmetic does not depend on the batch it is in (PCD_LT_NO_TAIL=1: the three tile-job phases of round 1)
-    const bool tail = std::getenv("PCD_LT_NO_TAIL") == nullptr;
-    if (tail) {
-        // PCD_LT_TAIL_DEC1=0: dec1 as a tile-job phase feeding the tail its split-K partial sums (the first round-2 form)
-        const bool tail_dec1 = std::getenv("PCD_LT_TAIL_DEC1") == nullptr || std::atoi(std::getenv("PCD_LT_TAIL_DEC1")) != 0;
-        const int ks = pick_ks(h->dec1c.cout, h->dec1c.cin);
-        if (!tail_dec1) P.ops[n++] = lt_gemm(pl->d2, 256, pl->z1, 128, h->t_dec1, 128, ks, LT_PARTIAL, pl->partial, nullptr, 0);
-        LtOp t = lt_norm(pl->partial, ks, h->dec1c.b, h->dec1c.gamma, h->dec1c.beta, 1, 128, nullptr);
+    // dec1 (from d2 and z1), its GroupNorm, output.0, output.2 and the update as ONE rows-per-CTA phase (latent_mk.cu, tail_phase), for
+    // every batch size so that a row's arithmetic does not depend on the batch it is in
+    {
+        LtOp t = lt_norm(nullptr, 0, h->dec1c.b, h->dec1c.gamma, h->dec1c.beta, 1, 128, nullptr);
         t.kind = LT_TAIL; t.W2 = h->out0T; t.b2 = h->out0.b; t.W3 = h->out2T; t.b3 = h->out2.b;
-        if (tail_dec1) { t.A0 = pl->d2; t.lda0 = 256; t.K0 = 256; t.A1 = pl->z1; t.lda1 = 128; t.K1 = 128; t.W = h->dec1cT; }
+        t.A0 = pl->d2; t.lda0 = 256; t.K0 = 256; t.A1 = pl->z1; t.lda1 = 128; t.K1 = 128; t.W = h->dec1cT;
         P.ops[n++] = t;
-    } else {
-        lt_layer(&P, &n, h->dec1c, h->t_dec1, pl->d2, 256, pl->z1, 128, pl->partial, pl->d1, 1);
-        P.ops[n++] = lt_gemm(pl->d1, 128, nullptr, 0, h->t_out0, 128, 1, LT_BIAS_RELU, pl->o0, h->out0.b, 0);
-        P.ops[n++] = lt_gemm(pl->o0, 128, nullptr, 0, h->t_out2, 256, 1, LT_FINAL, nullptr, h->out2.b, 0);
     }
     P.n_loop = n - P.n_pre;
-    if (const char* dbg = std::getenv("PCD_LT_MAXOPS")) {      // debugging aid: run only the first k phases
-        const int k = std::atoi(dbg);
-        if (k < P.n_pre) { P.n_pre = k; P.n_loop = 0; }
-        else if (k - P.n_pre < P.n_loop) P.n_loop = k - P.n_pre;
-    }
     CU(cudaMemcpy(pl->prog, &P, sizeof(P), cudaMemcpyHostToDevice));
     return 0;
 }
@@ -650,8 +624,9 @@ extern "C" int pcd_latent_sample_rows(pcd_latent* h, const float* sched, int32_t
 }
 
 // FoldingDecoder.forward (networks.py:1484-1509) on rows = (sample, grid point)
-// The folds on the tcgen05 split-precision GEMM (gemm_tc.cu, NP = 3, fp16 hi / lo planes): rows = B * 1024 is a multiple of 128.
-static int folding_decode_tc(pcd_latent* h, const float* z, float* out, int B, cudaStream_t s) {
+// The folds on the tcgen05 split-precision GEMM (gemm_tc.cu, NP = 3, fp16 hi / lo planes): rows = B * 1024 is a multiple of 128,
+// and its 8 B row blocks are always an even number for the CTA pairs.
+static int folding_decode(pcd_latent* h, const float* z, float* out, int B, cudaStream_t s) {
     const long long rows = static_cast<long long>(B) * 1024;
     const int P = h->upsample.cout;
     REQ(2 * rows < (1LL << 31), "FoldingDecoder: too many latents per call (decode in chunks)");
@@ -669,8 +644,9 @@ static int folding_decode_tc(pcd_latent* h, const float* z, float* out, int B, c
         if (make_tmap(&ta, h1, 2 * rows, 512, 512, 128) || make_tmap(&to, h3, 2 * rows, 512, 512, 32)) return 1;
         for (int f = 0; f < 2; ++f) {
             const pcd_latent::Fold& F = h->fold[f];
+            // per-sample bias: the latent columns of the fold's first conv (z is repeated over the grid, :1496)
             if (lin_op(h, nullptr, 0, F.wz, z, 256, nullptr, 0, bz, B, false, s, &n)) return 1;
-            CU(launch_fold_first(F.kin, f == 0 ? h->grid : o1, f == 0 ? 1024 : 0, F.wg, bz, rows, 1024, nullptr, h1, s)); ++n;
+            CU(launch_fold_first(F.kin, f == 0 ? h->grid : o1, f == 0 ? 1024 : 0, F.wg, bz, rows, 1024, h1, s)); ++n;
             if (make_tmap(&tb, F.wab16, 2 * 512, 512, 512, 128)) return 1;       // CTA pair: each CTA stages half of the 256-column tile
             TcGemmParams p{};
             p.num_m_blocks = static_cast<int>(rows / 128); p.num_n_blocks = 2; p.kb0 = 8; p.kb1 = 0;
@@ -680,48 +656,13 @@ static int folding_decode_tc(pcd_latent* h, const float* z, float* out, int B, c
             CU(launch_gemm_tc(256, EPI_STORE, 3, 2, 2, 1, ta, ta, tb, to, p, h->num_sms, s)); ++n;
             CU(launch_fold_tail16(h3, F.wbc.w, F.wbc.b, F.wc2, F.bc2, rows, 1024, f == 1 ? 1 : 0, f == 1 ? cm : o1, s)); ++n;
         }
-        if (lin_op(h, nullptr, 0, h->upsample, cm, 1024, nullptr, 0, U, 3 * B, false, s, &n)) return 1;
-        CU(launch_fold_transpose(U, B, P, out, s)); ++n;
-        return 0;
-    };
-    const int rc = run();
-    cudaFreeAsync(bz, s); cudaFreeAsync(h1, s); cudaFreeAsync(h3, s); cudaFreeAsync(o1, s); cudaFreeAsync(cm, s); cudaFreeAsync(U, s);
-    g_pcd_launches.fetch_add(n, std::memory_order_relaxed);
-    return rc;
-}
-
-static int folding_decode(pcd_latent* h, const float* z, float* out, int B, cudaStream_t s) {
-    if (h->fold_tc) return folding_decode_tc(h, z, out, B, s);      // 8 B row blocks of 128: always an even number for the CTA pairs
-    const long long rows = static_cast<long long>(B) * 1024;
-    const int P = h->upsample.cout;
-    REQ(rows / 64 <= 65535, "FoldingDecoder: at most 4095 latents per call (decode in chunks)");
-    float *bz = nullptr, *h1 = nullptr, *h3 = nullptr, *h5 = nullptr, *o1 = nullptr, *cm = nullptr, *U = nullptr;
-    CU(cudaMallocAsync(reinterpret_cast<void**>(&bz), sizeof(float) * B * 512, s));
-    CU(cudaMallocAsync(reinterpret_cast<void**>(&h1), sizeof(float) * rows * 512, s));
-    CU(cudaMallocAsync(reinterpret_cast<void**>(&h3), sizeof(float) * rows * 512, s));
-    CU(cudaMallocAsync(reinterpret_cast<void**>(&h5), sizeof(float) * rows * 3, s));
-    CU(cudaMallocAsync(reinterpret_cast<void**>(&o1), sizeof(float) * rows * 3, s));
-    CU(cudaMallocAsync(reinterpret_cast<void**>(&cm), sizeof(float) * rows * 3, s));
-    CU(cudaMallocAsync(reinterpret_cast<void**>(&U), sizeof(float) * 3 * B * P, s));
-    int n = 0;
-    auto run = [&]() -> int {
-        for (int f = 0; f < 2; ++f) {
-            const pcd_latent::Fold& F = h->fold[f];
-            // per-sample bias: the latent columns of the fold's first conv (z is repeated over the grid, :1496)
-            if (lin_op(h, nullptr, 0, F.wz, z, 256, nullptr, 0, bz, B, false, s, &n)) return 1;
-            CU(launch_fold_first(F.kin, f == 0 ? h->grid : o1, f == 0 ? 1024 : 0, F.wg, bz, rows, 1024, h1, nullptr, s)); ++n;
-            if (lin_op(h, nullptr, 0, F.wab, h1, 512, nullptr, 0, h3, static_cast<int>(rows), true, s, &n)) return 1;
-            if (lin_op(h, nullptr, 0, F.wbc, h3, 512, nullptr, 0, h5, static_cast<int>(rows), true, s, &n)) return 1;
-            CU(launch_fold_last(h5, F.wc2, F.bc2, rows, 1024, f == 1 ? 1 : 0, f == 1 ? cm : o1, s)); ++n;
-        }
         // upsample = Linear(1024 -> num_points) ACROSS the point axis of [B, 3, 1024] (:1507-1508)
         if (lin_op(h, nullptr, 0, h->upsample, cm, 1024, nullptr, 0, U, 3 * B, false, s, &n)) return 1;
         CU(launch_fold_transpose(U, B, P, out, s)); ++n;
         return 0;
     };
     const int rc = run();
-    cudaFreeAsync(bz, s); cudaFreeAsync(h1, s); cudaFreeAsync(h3, s); cudaFreeAsync(h5, s); cudaFreeAsync(o1, s);
-    cudaFreeAsync(cm, s); cudaFreeAsync(U, s);
+    cudaFreeAsync(bz, s); cudaFreeAsync(h1, s); cudaFreeAsync(h3, s); cudaFreeAsync(o1, s); cudaFreeAsync(cm, s); cudaFreeAsync(U, s);
     g_pcd_launches.fetch_add(n, std::memory_order_relaxed);
     return rc;
 }

@@ -44,6 +44,7 @@ namespace {
 constexpr int kG0 = 4;             // decoder_input grid edge
 constexpr int kC0 = 512;           // decoder_input channels
 constexpr int kVox = 32 * 32 * 32;
+constexpr int kTailLd = 32;        // channels per voxel row of decoder.12's input (dense 32-channel voxels)
 
 inline int pad64(int c) { return (c + 63) / 64 * 64; }
 
@@ -92,9 +93,6 @@ struct VPlan {
 
 struct pcd_vae3d {
     int precision = 0, device = 0, num_sms = 148, f16 = 0, planes = 1, latent = 256;
-    int grouped = 1;               // PCD_CONV_GROUP=0: every conv on the plain per-tap implicit GEMM (the A/B baseline)
-    int cluster = 2;               // PCD_CONV_CLUSTER=1: no CTA pairs in the grouped kernel
-    int final_ld = 64;             // channels per voxel row of decoder.12's input
     float *Win = nullptr, *bin = nullptr;     // decoder_input, rows permuted to channels-last: [(voxel * 512 + c)][latent]
     float *wf = nullptr, *bf = nullptr;       // decoder.12: [27][32] tap-major, [1]
     std::vector<ConvW> convs;
@@ -135,7 +133,7 @@ static int upload_conv(pcd_vae3d* h, const std::vector<float>& w, const std::vec
 static int pack_conv(pcd_vae3d* h, ConvW L, std::vector<Tap>& taps, const std::vector<float>& bias) {
     const int cin_kb = L.cin_pad / 64;
     const int bw = L.W, bh = bw > 0 && 128 % bw == 0 ? 128 / bw : 0;
-    bool can_group = h->grouped && L.cout_pad == 64 && bh >= 1 && bw % 8 == 0 && L.H % bh == 0;
+    bool can_group = L.cout_pad == 64 && bh >= 1 && bw % 8 == 0 && L.H % bh == 0;
     std::map<std::pair<int, int>, std::vector<int>> groups;          // (dd, dw) -> tap indices sorted by dh
     if (can_group) {
         for (size_t i = 0; i < taps.size(); ++i) groups[{taps[i].dd, taps[i].dw}].push_back(static_cast<int>(i));
@@ -309,8 +307,6 @@ extern "C" int pcd_vae3d_create(const pcd_named_tensor* tensors, int32_t n_tenso
     h->precision = precision; h->device = device; h->num_sms = prop.multiProcessorCount;
     h->f16 = (precision == PCD_PRECISION_F16 || precision == PCD_PRECISION_F16MIX) ? 1 : 0;
     h->planes = (precision == PCD_PRECISION_BF16X3 || precision == PCD_PRECISION_F16MIX) ? 2 : 1;
-    if (const char* c = std::getenv("PCD_CONV_GROUP")) h->grouped = std::atoi(c) != 0;
-    if (const char* c = std::getenv("PCD_CONV_CLUSTER")) h->cluster = std::atoi(c) == 2 ? 2 : 1;
 
     // ---- decoder_input (networks.py:2245, 2337-2338): row c * 64 + v of the reference -> row v * 512 + c (channels-last)
     {
@@ -343,11 +339,9 @@ extern "C" int pcd_vae3d_create(const pcd_named_tensor* tensors, int32_t n_tenso
         if (add_convT(h.get(), tt, "vae.decoder." + std::to_string(s.seqT), s.seqT, s.cin, s.cout, s.G)) return 1;
         if (res(s.seqR, s.cout, 2 * s.G, false)) return 1;
     }
-    // the 32-channel tail: dense 32-channel rows and voxel pairs when the grouped kernel runs, 64-padded channels otherwise
-    const bool dense32 = h->grouped != 0;
-    if (add_conv3(h.get(), tt, "vae.decoder.9", "", 9, 64, 32, 32, false, false, dense32)) return 1;
-    if (res(11, 32, 32, dense32)) return 1;
-    h->final_ld = dense32 ? 32 : 64;
+    // the 32-channel tail: dense 32-channel rows, decoder.11 on voxel pairs
+    if (add_conv3(h.get(), tt, "vae.decoder.9", "", 9, 64, 32, 32, false, false, true)) return 1;
+    if (res(11, 32, 32, true)) return 1;
     {
         const float *w, *b;
         if (!fetch(tt, "vae.decoder.12.weight", 27 * 32, &w, &err) || !fetch(tt, "vae.decoder.12.bias", 1, &b, &err)) return fail(err);
@@ -433,7 +427,7 @@ static int build_vplan(pcd_vae3d* h, int B, VPlan** out) {
             q.store5d = L.transposed ? 1 : 0; q.relu = 1; q.bias = L.bias;
             std::memcpy(q.gdw, L.gdw, 32); std::memcpy(q.gdh0, L.gdh0, 32); std::memcpy(q.gdd, L.gdd, 32);
             op.bn = 64;
-            op.cl = (h->cluster == 2 && q.num_m_blocks % 2 == 0) ? 2 : 1;
+            op.cl = q.num_m_blocks % 2 == 0 ? 2 : 1;
             const int bhh = q.bh + q.nt - 1;
             if (make_tmap5(&op.a0, pl->buf[src], L.cin_pad, L.W, L.H, L.D, nb, C, C * L.W, C * L.W * L.H, C * vox_in, q.bw, bhh, 1, 1))
                 return 1;
@@ -453,7 +447,6 @@ static int build_vplan(pcd_vae3d* h, int B, VPlan** out) {
             q.a_plane_rows = 0; q.b_plane_rows = PL == 2 ? L.cout_pad : 0; q.out_plane_rows = PL == 2 ? static_cast<int>(M) : 0;
             q.bias = L.bias; q.bias_sample_stride = 0; q.rows_per_sample = 1 << 30; q.relu = 1; q.f16 = h->f16;
             q.num_samples = Bp;
-            if (const char* d = std::getenv("PCD_DBG")) q.dbg = std::atoi(d) & 0xff;
             voxel_box(L.W, L.H, L.D, 128, box);
             if (make_tmap5(&op.a0, pl->buf[src], L.cin_pad, L.W, L.H, L.D, nb, C, C * L.W, C * L.W * L.H, C * vox_in, box[0], box[1], box[2], box[3]))
                 return 1;
@@ -511,8 +504,8 @@ static int launch_head(pcd_vae3d* h, VPlan* pl, const float* z, cudaStream_t s) 
 }
 
 static int launch_tail(pcd_vae3d* h, VPlan* pl, float* vox, cudaStream_t s) {
-    const long long plane_elems = static_cast<long long>(pl->Bpad) * kVox * h->final_ld;
-    LAUNCH(launch_vae3d_final_conv(pl->buf[pl->final_in], plane_elems, h->planes, h->f16, h->final_ld, 32, 32, 32, 32,
+    const long long plane_elems = static_cast<long long>(pl->Bpad) * kVox * kTailLd;
+    LAUNCH(launch_vae3d_final_conv(pl->buf[pl->final_in], plane_elems, h->planes, h->f16, kTailLd, 32, 32, 32, 32,
                                    static_cast<long long>(pl->B) * kVox, h->wf, h->bf, vox, s));
     return 0;
 }
@@ -550,7 +543,7 @@ extern "C" int pcd_vae3d_tap(pcd_vae3d* h, const float* z, int32_t B, int32_t se
     const long long vps = last < 0 ? 64 : pl->ops[last].L->out_rows;      // voxels per sample of the tapped activation
     const int creal = last < 0 ? kC0 : pl->ops[last].L->out_c;
     // channels per voxel row in memory (a voxel-pair layer stores [pair][64] = dense [voxel][32])
-    const int ld = last < 0 ? kC0 : (pl->ops[last].L->out_ld == 64 && creal == 32 && h->final_ld == 32 ? 32 : pl->ops[last].L->out_ld);
+    const int ld = last < 0 ? kC0 : (pl->ops[last].L->out_ld == 64 && creal == 32 ? 32 : pl->ops[last].L->out_ld);
     const void* src = last < 0 ? pl->buf[0] : pl->buf[pl->out_buf[last]];
     const long long rows = static_cast<long long>(B) * vps;
     REQ(count == rows * creal, "pcd_vae3d_tap: count must be B * G^3 * C of the tapped layer (channels-last)");

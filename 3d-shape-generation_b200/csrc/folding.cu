@@ -1,14 +1,14 @@
 // FoldingDecoder (reference networks.py:386-412, 1449-1509; PointNetVAE.decode :1579-1589): small kernels
-// around the fp32 GEMM of gemm_simt.cu.  Rows are (sample, grid point) pairs, 1024 grid points per sample.
+// around the tcgen05 GEMM of gemm_tc.cu.  Rows are (sample, grid point) pairs, 1024 grid points per sample.
 //
 // Algebra done at load time (api_latent.cu): a FoldingLayer is conv-ReLU-conv with NO activation after it, so the
 // second conv of one layer and the first conv of the next compose into one matrix; the latent columns of the first
 // conv of a fold multiply a per-sample constant and become a per-sample bias.  One fold is therefore
 //   h1 = relu(bias_z[b] + Wg * in[row])        in = grid point (K = 2) or fold1's output (K = 3)   (fold_first_kernel)
-//   h3 = relu(W_ab * h1 + b_ab)                512 x 512 GEMM      (tcgen05 split precision, gemm_tc.cu NP = 3; fp32 fallback: gemm_simt)
-//   h5 = relu(W_bc * h3 + b_bc)                3 x 512 GEMM                                         (fold_tail16_kernel / gemm_simt)
-//   out = W_c2 * h5 + b_c2                     3 x 3                                                (fold_tail16_kernel / fold_last_kernel)
-// Tensor-core form: h1 and h3 are fp16 hi + lo planes ([2 * rows][512], lo plane `rows` rows below; x = hi + lo to ~22 mantissa
+//   h3 = relu(W_ab * h1 + b_ab)                512 x 512 GEMM      (tcgen05 split precision, gemm_tc.cu NP = 3)
+//   h5 = relu(W_bc * h3 + b_bc)                3 x 512 GEMM        (fold_tail16_kernel)
+//   out = W_c2 * h5 + b_c2                     3 x 3               (fold_tail16_kernel)
+// h1 and h3 are fp16 hi + lo planes ([2 * rows][512], lo plane `rows` rows below; x = hi + lo to ~22 mantissa
 // bits) and the 512 x 512 GEMM runs D += hi*hi + hi*lo + lo*hi with fp32 accumulation: fp32-class results (measured 2e-6 relative
 // against the reference) at tensor-core rate.  96 % of the decoder's FLOPs.
 #include <cstdint>
@@ -20,11 +20,11 @@ namespace pcd {
 
 // out[row][c] = relu(bias[b][c] + sum_k W[c][k] * in[row_in][k]),  c < 512, 8 rows per CTA, 4 channels per thread.
 // in_mod > 0: row_in = row % in_mod (the shared 32 x 32 grid), otherwise row_in = row.
-// out16 != nullptr: write fp16 hi / lo planes (lo plane `plane_rows` rows below) instead of fp32
+// out16: fp16 hi / lo planes (lo plane `plane_rows` rows below)
 template <int KIN>
 __global__ void __launch_bounds__(128) fold_first_kernel(const float* __restrict__ in, int in_mod, const float* __restrict__ W,
                                                          const float* __restrict__ bias, int rows_per_sample,
-                                                         float* __restrict__ out, uint16_t* __restrict__ out16, long long plane_rows) {
+                                                         uint16_t* __restrict__ out16, long long plane_rows) {
     const int c0 = threadIdx.x * 4;
     float w[4][KIN];
 #pragma unroll
@@ -32,6 +32,7 @@ __global__ void __launch_bounds__(128) fold_first_kernel(const float* __restrict
 #pragma unroll
         for (int k = 0; k < KIN; ++k) w[j][k] = W[(c0 + j) * KIN + k];
     const long long row0 = static_cast<long long>(blockIdx.x) * 8;
+    uint16_t* __restrict__ lo16 = out16 + plane_rows * 512;
     const int b = static_cast<int>(row0 / rows_per_sample);          // 8 | rows_per_sample: one sample per CTA
     const float4 bz = *reinterpret_cast<const float4*>(bias + static_cast<long long>(b) * 512 + c0);
 #pragma unroll
@@ -48,19 +49,15 @@ __global__ void __launch_bounds__(128) fold_first_kernel(const float* __restrict
             for (int k = 0; k < KIN; ++k) v[j] = fmaf(w[j][k], x[k], v[j]);
             v[j] = fmaxf(v[j], 0.f);
         }
-        if (out16) {
-            const uint32_t h0 = pack16x2(v[0], v[1], 1), h1 = pack16x2(v[2], v[3], 1);
-            const float2 r0 = unpack16x2(h0, 1), r1 = unpack16x2(h1, 1);
-            *reinterpret_cast<uint2*>(out16 + row * 512 + c0) = make_uint2(h0, h1);
-            *reinterpret_cast<uint2*>(out16 + (row + plane_rows) * 512 + c0) =
-                make_uint2(pack16x2(v[0] - r0.x, v[1] - r0.y, 1), pack16x2(v[2] - r1.x, v[3] - r1.y, 1));
-        } else {
-            *reinterpret_cast<float4*>(out + row * 512 + c0) = make_float4(v[0], v[1], v[2], v[3]);
-        }
+        const uint32_t h0 = pack16x2(v[0], v[1], 1), h1 = pack16x2(v[2], v[3], 1);
+        const float2 r0 = unpack16x2(h0, 1), r1 = unpack16x2(h1, 1);
+        *reinterpret_cast<uint2*>(out16 + row * 512 + c0) = make_uint2(h0, h1);
+        *reinterpret_cast<uint2*>(lo16 + row * 512 + c0) =
+            make_uint2(pack16x2(v[0] - r0.x, v[1] - r0.y, 1), pack16x2(v[2] - r1.x, v[3] - r1.y, 1));
     }
 }
 
-// Tail of a fold on the tensor-core path: h3 arrives as fp16 hi / lo planes; h5 = relu(W_bc (hi + lo) + b_bc) (3 x 512, fp32
+// Tail of a fold: h3 arrives as fp16 hi / lo planes; h5 = relu(W_bc (hi + lo) + b_bc) (3 x 512, fp32
 // FMAs), out = W_c2 h5 + b_c2 (3 x 3).  One warp per row: a lane owns 16 of the 512 channels, shuffle reduction.
 __global__ void __launch_bounds__(256) fold_tail16_kernel(const uint16_t* __restrict__ h3, long long plane_rows, const float* __restrict__ Wbc,
                                                           const float* __restrict__ bbc, const float* __restrict__ Wc2,
@@ -107,26 +104,6 @@ __global__ void __launch_bounds__(256) fold_tail16_kernel(const uint16_t* __rest
     }
 }
 
-// out = W (3x3) * in[row] + b; channel_major = 0: out[row][3]; 1: out[b][c][n] with n = row % rows_per_sample
-__global__ void __launch_bounds__(256) fold_last_kernel(const float* __restrict__ in, const float* __restrict__ W,
-                                                        const float* __restrict__ bias, long long rows, int rows_per_sample,
-                                                        int channel_major, float* __restrict__ out) {
-    const long long row = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x;
-    if (row >= rows) return;
-    const float x0 = in[row * 3], x1 = in[row * 3 + 1], x2 = in[row * 3 + 2];
-    float v[3];
-#pragma unroll
-    for (int c = 0; c < 3; ++c) v[c] = fmaf(W[c * 3 + 2], x2, fmaf(W[c * 3 + 1], x1, fmaf(W[c * 3], x0, bias[c])));
-    if (channel_major) {
-        const long long b = row / rows_per_sample, n = row - b * rows_per_sample;
-#pragma unroll
-        for (int c = 0; c < 3; ++c) out[(b * 3 + c) * rows_per_sample + n] = v[c];
-    } else {
-#pragma unroll
-        for (int c = 0; c < 3; ++c) out[row * 3 + c] = v[c];
-    }
-}
-
 // U [B*3][P] (channel-major) -> out [B][P][3]
 __global__ void __launch_bounds__(256) fold_transpose_kernel(const float* __restrict__ U, int B, int P, float* __restrict__ out) {
     const long long i = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x;     // over B * P
@@ -137,11 +114,11 @@ __global__ void __launch_bounds__(256) fold_transpose_kernel(const float* __rest
 }
 
 cudaError_t launch_fold_first(int kin, const float* in, int in_mod, const float* W, const float* bias, long long rows,
-                              int rows_per_sample, float* out, void* out16, cudaStream_t s) {
+                              int rows_per_sample, void* out16, cudaStream_t s) {
     const int grid = static_cast<int>(rows / 8);
     uint16_t* o16 = static_cast<uint16_t*>(out16);
-    if (kin == 2) fold_first_kernel<2><<<grid, 128, 0, s>>>(in, in_mod, W, bias, rows_per_sample, out, o16, rows);
-    else if (kin == 3) fold_first_kernel<3><<<grid, 128, 0, s>>>(in, in_mod, W, bias, rows_per_sample, out, o16, rows);
+    if (kin == 2) fold_first_kernel<2><<<grid, 128, 0, s>>>(in, in_mod, W, bias, rows_per_sample, o16, rows);
+    else if (kin == 3) fold_first_kernel<3><<<grid, 128, 0, s>>>(in, in_mod, W, bias, rows_per_sample, o16, rows);
     else return cudaErrorInvalidValue;
     return cudaGetLastError();
 }
@@ -149,11 +126,6 @@ cudaError_t launch_fold_tail16(const void* h3, const float* Wbc, const float* bb
                                int rows_per_sample, int channel_major, float* out, cudaStream_t s) {
     fold_tail16_kernel<<<static_cast<unsigned>((rows + 7) / 8), 256, 0, s>>>(static_cast<const uint16_t*>(h3), rows, Wbc, bbc, Wc2, bc2, rows,
                                                                             rows_per_sample, channel_major, out);
-    return cudaGetLastError();
-}
-cudaError_t launch_fold_last(const float* in, const float* W, const float* bias, long long rows, int rows_per_sample,
-                             int channel_major, float* out, cudaStream_t s) {
-    fold_last_kernel<<<static_cast<int>((rows + 255) / 256), 256, 0, s>>>(in, W, bias, rows, rows_per_sample, channel_major, out);
     return cudaGetLastError();
 }
 cudaError_t launch_fold_transpose(const float* U, int B, int P, float* out, cudaStream_t s) {

@@ -379,10 +379,6 @@ __global__ void __launch_bounds__(256) zero_f32_kernel(float* __restrict__ p, lo
 cudaError_t launch_zero_f32(float* p, long long n, cudaStream_t stream) {
     return launch_pdl(zero_f32_kernel, dim3(static_cast<unsigned>((n + 255) / 256)), dim3(256), 0, stream, p, n);
 }
-bool pdl_enabled() {
-    const char* e = std::getenv("PCD_PDL");      // read per launch (launches are captured once per plan): tests flip it in-process
-    return e == nullptr || std::atoi(e) != 0;
-}
 cudaError_t launch_advance_step(int* step, cudaStream_t stream) {
     return launch_pdl(advance_step_kernel, dim3(1), dim3(1), 0, stream, step);
 }

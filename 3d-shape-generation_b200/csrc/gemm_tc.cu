@@ -204,14 +204,13 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
                     mbar_wait(&empty_bar[stage], phase ^ 1);
                     if constexpr (TWO) {
                         // both CTAs' loads are credited to the EVEN CTA's full barrier, which expects the bytes of the pair
-                        if (crank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * (A_STAGE + B_STAGE - (p.np2 ? kABytes : 0)));
+                        if (crank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * (A_STAGE + B_STAGE));
                         const uint32_t fb = mapa_shared(smem_u32(&full_bar[stage]), 0);
 #pragma unroll
                         for (int pl = 0; pl < PL; ++pl) {
                             uint8_t* da = sA + stage * A_STAGE + pl * kABytes;
                             const int arow = m_blk * kTileM + pl * p.a_plane_rows;
-                            if (pl == 1 && p.np2) {}                                   // two-pass layer: the A lo plane is never read
-                            else if (kb < p.kb0) tma_load_2d_2sm(da, &tmA0, fb, kb * kTileK, arow);
+                            if (kb < p.kb0) tma_load_2d_2sm(da, &tmA0, fb, kb * kTileK, arow);
                             else                 tma_load_2d_2sm(da, &tmA1, fb, (kb - p.kb0) * kTileK, arow);
                             tma_load_2d_2sm(sB + stage * B_STAGE + pl * B_BYTES, &tmB, fb, kb * kTileK,
                                             n_blk * BN + crank * (BN / 2) + pl * p.b_plane_rows);
@@ -219,14 +218,12 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
                         if (++stage == STAGES) { stage = 0; phase ^= 1; }
                         continue;
                     }
-                    mbar_arrive_expect_tx(&full_bar[stage], A_STAGE + B_STAGE - (p.np2 ? kABytes : 0));
+                    mbar_arrive_expect_tx(&full_bar[stage], A_STAGE + B_STAGE);
 #pragma unroll
                     for (int pl = 0; pl < PL; ++pl) {
                         uint8_t* da = sA + stage * A_STAGE + pl * kABytes;
                         const int arow = m_blk * kTileM + pl * p.a_plane_rows;
-                        if (pl == 1 && p.np2) {
-                            // two-pass layer (plain 2-D GEMMs only): the A lo plane is never read
-                        } else if (p.conv.ntaps > 0) {
+                        if (p.conv.ntaps > 0) {
                             // implicit-GEMM convolution: the tile's 128 voxels shifted by this k-block's tap
                             const ConvGeom& cg = p.conv;
                             const int v0 = m_blk * kTileM;
@@ -276,7 +273,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
                             tc_mma_2sm(d_tmem, da + 2 * k, db + 2 * k, IDESC, (kb | k) != 0 ? 1u : 0u);
                             if constexpr (NP == 3) {
                                 tc_mma_2sm(d_tmem, da + 2 * k, db + B_LO + 2 * k, IDESC, 1u);          // hi * lo
-                                if (!p.np2) tc_mma_2sm(d_tmem, da + A_LO + 2 * k, db + 2 * k, IDESC, 1u);          // lo * hi
+                                tc_mma_2sm(d_tmem, da + A_LO + 2 * k, db + 2 * k, IDESC, 1u);          // lo * hi
                             }
                             // c8: 32 e5m2 k-elements (32 bytes) of the byte planes per MMA: [Alo8 | Ahi8] . [Bhi8 | Blo8]
                             if constexpr (NP == 4) tc_mma_2sm_f8(d_tmem, da + A_LO + 2 * k, db + B_LO + 2 * k, IDESC8, 1u);
@@ -284,7 +281,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
                             tc_mma_bf16(d_tmem, da + 2 * k, db + 2 * k, IDESC, (kb | k) != 0 ? 1u : 0u);
                             if constexpr (NP == 3) {
                                 tc_mma_bf16(d_tmem, da + 2 * k, db + B_LO + 2 * k, IDESC, 1u);          // hi * lo
-                                if (!p.np2) tc_mma_bf16(d_tmem, da + A_LO + 2 * k, db + 2 * k, IDESC, 1u);          // lo * hi
+                                tc_mma_bf16(d_tmem, da + A_LO + 2 * k, db + 2 * k, IDESC, 1u);          // lo * hi
                             }
                         }
                     }
@@ -409,7 +406,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
                     uint8_t* stg_base = stage_out + (warp - 2) * (NBUF > 0 ? NBUF : 1) * 4096;
 #pragma unroll 1
                     for (int g2 = 0; g2 < BN / 64; ++g2) {
-                        if (p.dbg & 2) break;
                         uint32_t v0[32], v1[32];
                         tmem_ld_32x32(t_addr + g2 * 64, v0);
                         tmem_ld_32x32(t_addr + g2 * 64 + 32, v1);
@@ -454,7 +450,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
                                 else              { pk_lo[ch].z = l0; pk_lo[ch].w = l1; pk_lo[ch + 2].z = g0; pk_lo[ch + 2].w = g1; }
                             }
                         }
-                        if (p.dbg & 1) { if (pk[0].x == 0x12345678u && pk[7].w == 0x9abcdef0u) sb[0] = 0.f; continue; }
                         // the TMA store that used this staging tile NBUF stores ago must have finished READING it
                         uint8_t* stg = stg_base + sbuf * 4096;
                         if constexpr (NBUF > 1) { if (++sbuf == NBUF) sbuf = 0; }
@@ -465,9 +460,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
                             *reinterpret_cast<uint4*>(stg + lane * 128 + ((c ^ (lane & 7)) << 4)) = pk[c];
                         fence_proxy_async_smem();
                         __syncwarp();
-                        if (lane == 0 && !(p.dbg & 4)) {
+                        if (lane == 0) {
                             if (p.conv.store5d) conv_store_5d(&tmOut, stg, p.conv, n_blk * BN + g2 * 64, m_blk * kTileM + q * 32, 0);
-                            else if (p.dbg & 8) tma_store_2d(&tmOut, stg, g2 * 64, q * 32);   // timing experiment: L2-only write traffic
                             else tma_store_2d(&tmOut, stg, n_blk * BN + g2 * 64, m_blk * kTileM + q * 32);
                             tma_store_commit();
                         }
@@ -618,7 +612,7 @@ static cudaError_t launch_ew(const CUtensorMap& a0, const CUtensorMap& a1, const
     attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl_enabled() ? 2 : 1;
+    cfg.attrs = attr; cfg.numAttrs = 2;
     if (p.f16) return cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BN, EPI, NP, CL, OP, TWO, 1, EW>, a0, a1, b, o, p);
     if constexpr (NP == 4 || OP == 3) return cudaErrorInvalidValue;
     else return cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BN, EPI, NP, CL, OP, TWO, 0, EW>, a0, a1, b, o, p);

@@ -11,7 +11,7 @@
 // Arithmetic: every Linear is a set of 128 x 64 x K tile jobs on tcgen05 (kind::tf32, fp32 accumulators in TMEM) with the
 // 3xTF32 split (x = hi + lo; D += lo*hi + hi*lo + hi*hi): < 2^-20 relative per product, i.e. the results sit inside the fp32
 // parity bound (2e-5 per forward) that the CUDA-core path was held to.  kind::tf32 ignores the 13 low mantissa bits of its
-// fp32 containers (measured, tools/dbg_trunc.py), so a value as loaded IS its hi operand and only lo = x - trunc(x) is computed.
+// fp32 containers (measured, DESIGN.md §5.4), so a value as loaded IS its hi operand and only lo = x - trunc(x) is computed.
 // Operands stay fp32 in global memory (weights 76 MB: L2 resident).
 //   * Weights are stored tile-major and pre-swizzled, so a 64 x 32 (or 128 x 32) tile is ONE 8 / 16 KB bulk copy (cp.async.bulk, mbarrier
 //     complete_tx) that lands in the canonical SWIZZLE_128B K-major layout; warps 4-7 write the lo plane next to it.
@@ -24,7 +24,7 @@
 // vectorised epilogues + one-round-trip GroupNorm loads + cheap split 178; program in shared memory + release-red barrier
 // 162; no hi write-back 151; activations through TMEM 140; 128-column tiles for the three big layers + ONE call site for the
 // phase interpreter (the code is 150 KB, far beyond the instruction cache: halving it sped up every phase) 138; one chunk per split for the small layers 136.  The per-phase
-// trace (PCD_LT_TRACE, tools/trace_latent.py) and the PCD_LT_DBG experiments are what found each of these.  Tried and
+// trace (PCD_LT_TRACE, tools/trace_latent.py) and timing experiments without the split or the MMAs are what found each of these.  Tried and
 // rejected: rows straight into registers (32 lines per load instruction: 160), deeper rings (NST 6 / PF 4: 143), A and W work
 // shared by all 8 warps (157), two-level grid barrier, more than 168 registers (9 warps: one scheduler holds 3 of them),
 // starting the next GEMM phase's first weight tiles before the barrier (145.7 against 139.4 without, same build and box),
@@ -112,7 +112,6 @@ struct Pipe {
     uint32_t tmem;          // accumulator: 128 lanes x 64 fp32 columns
     uint32_t gc;            // chunks issued so far (uniform across the CTA): stage = gc % NST, use = gc / NST
     uint32_t jobs;          // tile jobs done so far by this CTA
-    int dbg;                // PCD_LT_DBG timing experiments (results are garbage): 1 zero lo planes (no split arithmetic), 8 no MMAs
 };
 
 
@@ -167,7 +166,6 @@ __device__ void gemm_item_mma(const LtOp& op, Pipe& pp) {
         const uint32_t w_hi = lo_base + ((st * STAGE * 4) >> 4), w_lo = w_hi + ((W_PLANE * 4) >> 4);
 #pragma unroll
         for (int k = 0; k < BK / 8; ++k) {
-            if (pp.dbg & 8) break;
             tc_mma_tf32_ts(pp.tmem, a_lo + 8 * k, hi_bits | (w_hi + 2 * k), idesc, (ci | k) ? 1u : 0u);     // small terms first
             tc_mma_tf32_ts(pp.tmem, a_hi + 8 * k, hi_bits | (w_lo + 2 * k), idesc, 1u);
             tc_mma_tf32_ts(pp.tmem, a_hi + 8 * k, hi_bits | (w_hi + 2 * k), idesc, 1u);
@@ -186,7 +184,7 @@ __device__ void gemm_item_mma(const LtOp& op, Pipe& pp) {
 //              registers, one 128-byte line per lane, was slower: 32 lines per load instruction.)
 //   warps 4-7: one thread issues the 8 KB weight-tile bulk copies (PF chunks ahead); all wait for the tile and write its lo plane.
 // The 3xTF32 split: tcgen05 kind::tf32 IGNORES the 13 low mantissa bits of its fp32 containers (measured: masking them first
-// gives bit-identical results, tools/dbg_trunc.py), so the loaded value already is the hi operand (hi = trunc(x)) and only
+// gives bit-identical results, DESIGN.md §5.4), so the loaded value already is the hi operand (hi = trunc(x)) and only
 // lo = x - trunc(x) -- exact in fp32, truncated again by the MMA -- has to be produced.  x - (hi + lo) < 2^-20 |x|.
 template <int BN_>
 __device__ void gemm_item(const LtOp& op, const LatentCall& c, const StepCtx& cx, int rows, int m_tile, int n_tile, int split,
@@ -235,7 +233,7 @@ __device__ void gemm_item(const LtOp& op, const LatentCall& c, const StepCtx& cx
 #pragma unroll
                 for (int q = 0; q < 4; ++q) {
                     hi[4 * j + q] = __float_as_uint(x[q]);
-                    lo[4 * j + q] = (pp.dbg & 1) ? 0u : __float_as_uint(x[q] - __uint_as_float(__float_as_uint(x[q]) & 0xffffe000u));
+                    lo[4 * j + q] = __float_as_uint(x[q] - __uint_as_float(__float_as_uint(x[q]) & 0xffffe000u));
                 }
             }
             if (g >= NST) mbar_wait(&pp.mma_done[st], ((g / NST) - 1) & 1);     // the MMAs that read this TMEM stage have completed
@@ -281,7 +279,6 @@ __device__ void gemm_item(const LtOp& op, const LatentCall& c, const StepCtx& cx
                     l.y = __uint_as_float(x[i].y) - __uint_as_float(x[i].y & 0xffffe000u);
                     l.z = __uint_as_float(x[i].z) - __uint_as_float(x[i].z & 0xffffe000u);
                     l.w = __uint_as_float(x[i].w) - __uint_as_float(x[i].w & 0xffffe000u);
-                    if (pp.dbg & 1) l = make_float4(0.f, 0.f, 0.f, 0.f);
                     l4[wt + i * 128] = l;
                 }
             }
@@ -357,6 +354,8 @@ __device__ void gemm_item(const LtOp& op, const LatentCall& c, const StepCtx& cx
 #pragma unroll
         for (int j = 0; j < 32; ++j) v[j] = v[j] / (1.f + expf(-v[j]));
     }
+    // No program emits LT_FINAL any more (the tail phase runs the sampler update), but without this epilogue ptxas spills the
+    // phase loop's state of latent_mk_kernel (56 bytes at the 168-register cap), so it stays.
     if (op.epi != LT_FINAL) {
         float4* dst = reinterpret_cast<float4*>(op.out + static_cast<long long>(r) * op.ldo + nb);
 #pragma unroll
@@ -521,7 +520,7 @@ __device__ __forceinline__ void final_update_one(const LatentCall& c, const Step
 // LT_TAIL: for small batches the last three phases (dec1's GroupNorm, output.0, output.2 + sampler update: networks.py:1083-1086,
 // diffusion.py:586-606 / 637-645) are 49 k MACs per row behind three grid barriers and two tile-job pipelines that have nothing
 // to chew on (2 and 4 busy CTAs, 8 and 10 us at batch 128).  Rows are independent here, so ONE phase does them on CUDA cores, a few rows per CTA:
-// fixed-order split-K reduce + GroupNorm(8, 128) + ReLU, a 128 x 128 and a 128 x 256 matrix-vector product against transposed
+// dec1 itself (a 384 x 128 matrix-vector product) + GroupNorm(8, 128) + ReLU, a 128 x 128 and a 128 x 256 matrix-vector product against transposed
 // weights (coalesced, L2-resident, 192 KB) with 8 independent accumulators per thread, then the update.  fp32 FMAs throughout.
 // RT rows per CTA pass share every weight load (RT = ceil(rows / grid) rounded up to 1, 2 or 4); a row's own arithmetic -- order of
 // every sum included -- does not depend on RT or on which rows it is grouped with, so results stay batch independent.
@@ -532,56 +531,48 @@ template <int RT>
 __device__ void tail_rows(const LtOp& op, const LatentCall& c, const StepCtx& cx, int rows, float (*sh_h)[128], float (*sh_a)[128],
                           float* sh_p /* [8][RT][128] or [4][RT][256] */, float* sx /* [RT][384], the idle tile-job ring */) {
     const int tid = threadIdx.x;
-    const bool own_dec1 = op.K0 > 0;       // dec1 = Linear(cat([d2, refine1(z1)])) computed here (W = composed weights [384][128]^T)
     for (int r0 = blockIdx.x * RT; r0 < rows; r0 += gridDim.x * RT) {
-        if (own_dec1) {
-            for (int i = tid; i < RT * 96; i += NTHREADS) {
-                const int rr = i / 96, q = i - rr * 96, r = r0 + rr;
-                float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (r < rows)
-                    v = q < 64 ? __ldcg(reinterpret_cast<const float4*>(op.A0 + static_cast<long long>(r) * 256) + q)
-                               : __ldcg(reinterpret_cast<const float4*>(op.A1 + static_cast<long long>(r) * 128) + (q - 64));
-                reinterpret_cast<float4*>(sx)[i] = v;
-            }
-            __syncthreads();
-            if (tid < 256) {                                     // thread = (k group of 48, four outputs)
-                const int og = tid & 31, kg = tid >> 5;
-                const float4* w = reinterpret_cast<const float4*>(op.W + static_cast<long long>(kg * 48) * 128) + og;
-                float4 acc[RT];
-#pragma unroll
-                for (int i = 0; i < RT; ++i) acc[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-                for (int kh = 0; kh < 3; ++kh) {
-                    float4 wv[16];
-#pragma unroll
-                    for (int k = 0; k < 16; ++k) wv[k] = __ldg(w + (kh * 16 + k) * 32);
-#pragma unroll
-                    for (int i = 0; i < RT; ++i)
-#pragma unroll
-                        for (int k = 0; k < 16; ++k) {
-                            const float x = sx[i * 384 + kg * 48 + kh * 16 + k];
-                            acc[i].x = fmaf(wv[k].x, x, acc[i].x); acc[i].y = fmaf(wv[k].y, x, acc[i].y);
-                            acc[i].z = fmaf(wv[k].z, x, acc[i].z); acc[i].w = fmaf(wv[k].w, x, acc[i].w);
-                        }
-                }
-#pragma unroll
-                for (int i = 0; i < RT; ++i) *reinterpret_cast<float4*>(sh_p + (kg * RT + i) * 128 + 4 * og) = acc[i];
-            }
-            __syncthreads();
+        // dec1 = Linear(cat([d2, refine1(z1)])) (W = composed weights [384][128]^T)
+        for (int i = tid; i < RT * 96; i += NTHREADS) {
+            const int rr = i / 96, q = i - rr * 96, r = r0 + rr;
+            float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (r < rows)
+                v = q < 64 ? __ldcg(reinterpret_cast<const float4*>(op.A0 + static_cast<long long>(r) * 256) + q)
+                           : __ldcg(reinterpret_cast<const float4*>(op.A1 + static_cast<long long>(r) * 128) + (q - 64));
+            reinterpret_cast<float4*>(sx)[i] = v;
         }
+        __syncthreads();
+        if (tid < 256) {                                     // thread = (k group of 48, four outputs)
+            const int og = tid & 31, kg = tid >> 5;
+            const float4* w = reinterpret_cast<const float4*>(op.W + static_cast<long long>(kg * 48) * 128) + og;
+            float4 acc[RT];
+#pragma unroll
+            for (int i = 0; i < RT; ++i) acc[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+            for (int kh = 0; kh < 3; ++kh) {
+                float4 wv[16];
+#pragma unroll
+                for (int k = 0; k < 16; ++k) wv[k] = __ldg(w + (kh * 16 + k) * 32);
+#pragma unroll
+                for (int i = 0; i < RT; ++i)
+#pragma unroll
+                    for (int k = 0; k < 16; ++k) {
+                        const float x = sx[i * 384 + kg * 48 + kh * 16 + k];
+                        acc[i].x = fmaf(wv[k].x, x, acc[i].x); acc[i].y = fmaf(wv[k].y, x, acc[i].y);
+                        acc[i].z = fmaf(wv[k].z, x, acc[i].z); acc[i].w = fmaf(wv[k].w, x, acc[i].w);
+                    }
+            }
+#pragma unroll
+            for (int i = 0; i < RT; ++i) *reinterpret_cast<float4*>(sh_p + (kg * RT + i) * 128 + 4 * og) = acc[i];
+        }
+        __syncthreads();
         if (tid < 128) {
 #pragma unroll
             for (int i = 0; i < RT; ++i) {
                 const int r = r0 + i;
-                float v = 0.f;
-                if (own_dec1) {
-                    v = __ldg(bias_row(op, r < rows ? r : 0, cx) + tid);
+                float v = __ldg(bias_row(op, r < rows ? r : 0, cx) + tid);
 #pragma unroll
-                    for (int kg = 0; kg < 8; ++kg) v += sh_p[(kg * RT + i) * 128 + tid];          // fixed order
-                } else if (r < rows) {
-                    v = __ldg(bias_row(op, r, cx) + tid);
-                    for (int sp = 0; sp < op.nsplit; ++sp) v += __ldcg(op.partial + (static_cast<long long>(sp) * rows + r) * 128 + tid);
-                }
+                for (int kg = 0; kg < 8; ++kg) v += sh_p[(kg * RT + i) * 128 + tid];          // fixed order
                 float s1 = v;                                    // GroupNorm(8, 128): 16 consecutive channels = half a warp
 #pragma unroll
                 for (int o = 8; o; o >>= 1) s1 += __shfl_xor_sync(0xffffffffu, s1, o);
@@ -833,7 +824,7 @@ __device__ void run_op(const LtOp& op, const LatentCall& c, const StepCtx& cx, i
 
 __global__ void __launch_bounds__(NTHREADS, 1) latent_mk_kernel(const LtProgram* __restrict__ prog, const LatentCall* __restrict__ callp,
                                                            int S, int R, int forward, unsigned* bar,
-                                                           unsigned long long* trace, int dbg) {
+                                                           unsigned long long* trace) {
     extern __shared__ __align__(16) unsigned char lt_smem_raw[];
     __shared__ __align__(8) uint64_t mma_done[NST];
     __shared__ __align__(8) uint64_t w_full[NST];
@@ -848,7 +839,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) latent_mk_kernel(const LtProgram*
     pp.ready = ready;
     pp.acc_free = &acc_free;
     pp.jobs = 0;
-    pp.dbg = dbg;
     pp.gc = 0;
     if (threadIdx.x == 0) {
         for (int i = 0; i < NST; ++i) { mbar_init(&mma_done[i], 1); mbar_init(&w_full[i], 1); mbar_init(&ready[i], NWORK / 32); }
@@ -965,9 +955,7 @@ cudaError_t launch_latent_mk(const LtProgram* prog, const LatentCall* call, int 
         if (e != cudaSuccess) return e;
         cudaMemset(trace, 0, sizeof(unsigned long long) * grid * 40 * 3);
     }
-    const char* dbg_env = std::getenv("PCD_LT_DBG");
-    int dbg = dbg_env ? std::atoi(dbg_env) : 0;
-    void* args[] = {&prog, &call, &S, &R, &forward, &bar, &trace, &dbg};
+    void* args[] = {&prog, &call, &S, &R, &forward, &bar, &trace};
     e = cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(latent_mk_kernel), dim3(grid), dim3(NTHREADS), args, kLtSmemBytes, stream);
     if (trace) {
         cudaStreamSynchronize(stream);

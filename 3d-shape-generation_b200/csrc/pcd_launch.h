@@ -8,9 +8,7 @@
 
 namespace pcd {
 
-// Programmatic dependent launch (see pcd_ptx.cuh): PCD_PDL=0 turns the attribute off (the kernels' griddepcontrol instructions are
-// then no-ops) for A/B timing.
-bool pdl_enabled();
+// Programmatic dependent launch (see pcd_ptx.cuh)
 template <typename... KArgs, typename... Args>
 cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args) {
     cudaLaunchConfig_t cfg{};
@@ -18,7 +16,7 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.attrs = attr; cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 cudaError_t launch_zero_f32(float* p, long long n, cudaStream_t stream);
@@ -73,11 +71,9 @@ cudaError_t launch_sinkhorn_cost(const float4* Q, const float4* T, const float* 
                                  const unsigned* cmax_bits, float lambda, float scaling, float* partial, float* emd, cudaStream_t s);
 
 cudaError_t launch_fold_first(int kin, const float* in, int in_mod, const float* W, const float* bias, long long rows,
-                              int rows_per_sample, float* out, void* out16, cudaStream_t s);
+                              int rows_per_sample, void* out16, cudaStream_t s);
 cudaError_t launch_fold_tail16(const void* h3, const float* Wbc, const float* bbc, const float* Wc2, const float* bc2, long long rows,
                                int rows_per_sample, int channel_major, float* out, cudaStream_t s);
-cudaError_t launch_fold_last(const float* in, const float* W, const float* bias, long long rows, int rows_per_sample,
-                             int channel_major, float* out, cudaStream_t s);
 cudaError_t launch_fold_transpose(const float* U, int B, int P, float* out, cudaStream_t s);
 
 cudaError_t launch_groupnorm_relu(float* y, const float* partial, int nsplit, const float* bias, const float* gamma, const float* beta,

@@ -73,8 +73,8 @@ struct LtOp {
     const float* partial; int nsplit;
     const float* gamma; const float* beta;
     int act, C;
-    // LT_TAIL (small batches): the last GroupNorm + output.0 + ReLU + output.2 + the sampler update as ONE row-per-CTA phase on
-    // CUDA cores (weights transposed [in][out]); partial / nsplit / bias / gamma / beta describe dec1 as in LT_NORM
+    // LT_TAIL: dec1 + its GroupNorm + output.0 + ReLU + output.2 + the sampler update as ONE row-per-CTA phase on CUDA cores
+    // (weights transposed [in][out]); A0 / A1 / W = dec1's inputs and composed weights, bias / gamma / beta its GroupNorm as in LT_NORM
     const float* W2; const float* b2;    // output.0  [128][128]^T
     const float* W3; const float* b3;    // output.2  [128][256]^T
     // LT_HEAD (the first two layers as ONE row-per-CTA phase on CUDA cores): W2 = enc1's z columns [256][128]^T with bias (one row
@@ -176,11 +176,7 @@ struct TcGemmParams {
     int epi_warps;      // EPI_STORE: 8 = two epilogue warps per TMEM lane quarter on 32-column sub-groups (tmOut box 32 x 32, SWIZZLE_64B;
                         // plain 2-D stores only); 0 / 4 = one warp per quarter on 64-column groups (tmOut box 64 x 32, SWIZZLE_128B)
     int tile_order;     // STORE / FINAL tile schedule: 0 = a cluster keeps its row block across the weight tiles, 1 = n fastest (gemm_tc.cu)
-    int np2;            // split-precision layer run as TWO passes (Ahi*Bhi + Ahi*Blo): the activation's lo plane is neither loaded nor
-                        // multiplied -- the layer sees fp16-rounded activations and full-precision weights
     int f16;            // 16-bit operand/activation format: 0 = bf16, 1 = fp16 (values saturate at +-65504); selects the kernel instantiation
-    int dbg;            // PCD_DBG timing experiments only: bit 0 skips the output store path, bit 1 skips the epilogue TMEM reads,
-                        // bit 2 stages in smem but skips the TMA store, bit 3 stores every tile to the same (L2-resident) location
     const CallArgs* call;   // EPI_FINAL: per-call arguments live in device memory (graph-invariant)
 };
 

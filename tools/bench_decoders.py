@@ -1,6 +1,6 @@
 """Throughput of the decoders and of the Sinkhorn EMD next to the point / latent loops (tracked numbers the round-1 review asked
-for): FoldingDecoder (PointNetVAE.decode, networks.py:1449-1509) on the tcgen05 split-precision path vs the fp32 CUDA-core
-path (PCD_FOLD_SIMT=1, one subprocess each), and earth_mover_distance_gpu (metrics.py:94-158) on 2048-point clouds."""
+for): FoldingDecoder (PointNetVAE.decode, networks.py:1449-1509) on the tcgen05 split-precision path, and
+earth_mover_distance_gpu (metrics.py:94-158) on 2048-point clouds (one subprocess each)."""
 import json
 import os
 import subprocess
@@ -39,7 +39,7 @@ def folding():
         z = torch.randn(B, 256, generator=g).cuda()
         ms, out = timed(lambda: vae.decode(z), 5)
         flops = 2.0 * B * 1024 * (2 * (512 * 512 + 3 * 512 + 512 * 3) + 9 * 2) + 2.0 * 3 * B * 1024 * NP
-        print(json.dumps({"what": "FoldingDecoder.decode -> 2048 pts", "path": "fp32 CUDA cores" if os.environ.get("PCD_FOLD_SIMT") else "tcgen05 fp16 hi+lo, 3 passes",
+        print(json.dumps({"what": "FoldingDecoder.decode -> 2048 pts", "path": "tcgen05 fp16 hi+lo, 3 passes",
                           "batch": B, "ms": ms, "latents_per_s": B / ms * 1e3, "algorithmic_tflops": flops / ms / 1e9,
                           "rel_l2_vs_oracle_b2": err, "finite": bool(torch.isfinite(out).all())}), flush=True)
 
@@ -62,5 +62,4 @@ if __name__ == "__main__":
         {"folding": folding, "emd": emd}[sys.argv[1]]()
     else:
         subprocess.run([sys.executable, __file__, "folding"], timeout=600)
-        subprocess.run([sys.executable, __file__, "folding"], env=dict(os.environ, PCD_FOLD_SIMT="1"), timeout=600)
         subprocess.run([sys.executable, __file__, "emd"], timeout=600)

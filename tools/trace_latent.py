@@ -3,12 +3,9 @@ first CTA entering it to the last CTA leaving its barrier, the longest / mean pe
 import os, sys, collections
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-NAMES_R1 = ["enc1 G", "enc1 N", "enc2 G", "enc2 N", "enc3 G", "enc3 N", "enc4 G", "enc4 N", "gf0 G", "gf0 N", "gf3 G", "gf3 N",
-            "dec4 G", "dec4 N", "dec3 G", "dec3 N", "dec2 G", "dec2 N", "dec1 G", "dec1 N", "out0", "out2+update"]
-# round 2 program: enc1 + enc2 are the head phase, dec1 + output.0 + output.2 + update the tail phase
-NAMES_R2 = ["head (enc1+enc2)", "enc3 G", "enc3 N", "enc4 G", "enc4 N", "gf0 G", "gf0 N", "gf3 G", "gf3 N",
-            "dec4 G", "dec4 N", "dec3 G", "dec3 N", "dec2 G", "dec2 N", "tail (dec1+out0+out2+update)"]
-NAMES = NAMES_R1 if (os.environ.get("PCD_LT_NO_HEAD") and os.environ.get("PCD_LT_NO_TAIL")) else NAMES_R2
+# enc1 + enc2 are the head phase, dec1 + output.0 + output.2 + update the tail phase
+NAMES = ["head (enc1+enc2)", "enc3 G", "enc3 N", "enc4 G", "enc4 N", "gf0 G", "gf0 N", "gf3 G", "gf3 N",
+         "dec4 G", "dec4 N", "dec3 G", "dec3 N", "dec2 G", "dec2 N", "tail (dec1+out0+out2+update)"]
 import torch
 import pcd_b200
 from oracle import pointdiff_oracle as O
