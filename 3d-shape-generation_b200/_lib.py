@@ -16,7 +16,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("PCD_LIB_PATH") or os.path.join(_HERE, "libpcd_b200.so")   # PCD_LIB_PATH: A/B-compare two builds on one box
 CSRC = os.path.join(_HERE, "csrc")
-SOURCES = ["api.cu", "api_latent.cu", "gemm_tc.cu", "gemm_simt.cu", "chamfer.cu", "emd.cu", "latent.cu", "latent_mk.cu", "chain_tc.cu", "folding.cu", "api_vae3d.cu", "vae3d.cu", "conv3d_tc.cu"]
+SOURCES = ["api.cu", "api_latent.cu", "gemm_tc.cu", "gemm_simt.cu", "chamfer.cu", "emd.cu", "emd_exact.cu", "latent.cu", "latent_mk.cu", "chain_tc.cu", "folding.cu", "api_vae3d.cu", "vae3d.cu", "conv3d_tc.cu"]
 
 PRECISION = {"bf16": 0, "fp32": 1, "bf16x3": 2, "f16": 3, "f16mix": 4}
 SCHED_ROW = 8
@@ -111,6 +111,8 @@ _SIGNATURES = {
                                      C.c_void_p]),
     "pcd_sinkhorn_emd": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_float, C.c_int32,
                                    C.c_float, C.c_void_p, C.POINTER(C.c_int32), C.c_void_p]),
+    "pcd_emd_exact": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_void_p, C.c_void_p,
+                                C.c_void_p]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 
@@ -327,3 +329,20 @@ def sinkhorn_emd(x: torch.Tensor, y: torch.Tensor, epsilon: float = 1e-2, thresh
     check(lib().pcd_sinkhorn_emd(x.data_ptr(), y.data_ptr(), B, N, y.shape[1], epsilon, thresh, max_iter, scaling,
                                  emd.data_ptr(), C.byref(iters), stream_ptr(x.device)))
     return emd, int(iters.value)
+
+
+def emd_exact(x: torch.Tensor, y: torch.Tensor, scaling: float = 1.0, return_assignment: bool = False):
+    """Per-pair exact EMD (reference metrics.py:49-92) -> emd[B] on the device and, with return_assignment, the matched y index
+    of every x as int32 [B, N] (-1: unmatched)."""
+    _require_cuda(x, "x")
+    _require_cuda(y, "y")
+    x = x.to(torch.float32).contiguous()
+    y = y.to(torch.float32).contiguous()
+    B, N, _ = x.shape
+    assert y.shape[0] == B, "batch sizes must be the same"
+    emd = torch.empty(B, device=x.device, dtype=torch.float32)
+    assign = torch.empty(B, N, device=x.device, dtype=torch.int32) if return_assignment else None
+    if B > 0:
+        check(lib().pcd_emd_exact(x.data_ptr(), y.data_ptr(), B, N, y.shape[1], scaling, emd.data_ptr(),
+                                  assign.data_ptr() if return_assignment else None, stream_ptr(x.device)))
+    return (emd, assign) if return_assignment else emd

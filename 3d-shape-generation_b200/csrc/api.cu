@@ -1122,3 +1122,35 @@ extern "C" int pcd_sinkhorn_emd(const float* x, const float* y, int32_t B, int32
     cudaFreeAsync(xn, s); cudaFreeAsync(yn, s); cudaFreeAsync(work, s);
     return rc;
 }
+
+// ------------------------------------------------------------------------------------------
+// Exact EMD (metrics.py:49-92): auction assignment per pair, emd_exact.cu
+// ------------------------------------------------------------------------------------------
+extern "C" int pcd_emd_exact(const float* x, const float* y, int32_t B, int32_t N, int32_t M, float scaling, float* emd,
+                             int32_t* assign_xy, void* stream) {
+    REQ(x && y && emd, "null argument");
+    REQ(B > 0 && N > 0 && M > 0, "B, N, M must be positive");
+    REQ(B <= 65535, "at most 65535 pairs per call");
+    REQ(emd_exact_fits(N, M), "exact EMD supports at most 4096 points per cloud (N = " + std::to_string(N) + ", M = " +
+                                  std::to_string(M) + ")");
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    float4 *xn = nullptr, *yn = nullptr;
+    int* err = nullptr;
+    CU(cudaMallocAsync(reinterpret_cast<void**>(&xn), sizeof(float4) * B * N, s));
+    CU(cudaMallocAsync(reinterpret_cast<void**>(&yn), sizeof(float4) * B * M, s));
+    CU(cudaMallocAsync(reinterpret_cast<void**>(&err), sizeof(int), s));
+    auto run = [&]() -> int {
+        CU(cudaMemsetAsync(err, 0, sizeof(int), s));
+        LAUNCH(launch_cloud_norm(x, B, N, xn, s));
+        LAUNCH(launch_cloud_norm(y, B, M, yn, s));
+        LAUNCH(launch_emd_exact(xn, yn, B, N, M, scaling, emd, assign_xy, err, s));
+        int e = 0;
+        CU(cudaMemcpyAsync(&e, err, sizeof(int), cudaMemcpyDeviceToHost, s));
+        CU(cudaStreamSynchronize(s));      // the round-cap flag is the only thing read back
+        REQ(e == 0, "exact EMD: an auction phase exceeded its round cap (the affected pairs are NaN)");
+        return 0;
+    };
+    const int rc = run();
+    cudaFreeAsync(xn, s); cudaFreeAsync(yn, s); cudaFreeAsync(err, s);
+    return rc;
+}

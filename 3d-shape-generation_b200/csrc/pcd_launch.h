@@ -1,4 +1,4 @@
-// Launcher prototypes (defined in gemm_tc.cu, gemm_simt.cu, chamfer.cu).
+// Launcher prototypes (defined in gemm_tc.cu, gemm_simt.cu, chamfer.cu, emd.cu, emd_exact.cu).
 #pragma once
 #include <cstdlib>
 #include <utility>
@@ -69,6 +69,10 @@ cudaError_t launch_sinkhorn_half(const float4* Q, const float4* T, const float* 
                                  cudaStream_t s);
 cudaError_t launch_sinkhorn_cost(const float4* Q, const float4* T, const float* alpha, const float* beta, int pairs, int Nq, int Nt,
                                  const unsigned* cmax_bits, float lambda, float scaling, float* partial, float* emd, cudaStream_t s);
+
+bool emd_exact_fits(int N, int M);
+cudaError_t launch_emd_exact(const float4* X, const float4* Y, int pairs, int N, int M, float scaling, float* emd, int* assign_xy,
+                             int* err, cudaStream_t s);
 
 cudaError_t launch_fold_first(int kin, const float* in, int in_mod, const float* W, const float* bias, long long rows,
                               int rows_per_sample, void* out16, cudaStream_t s);

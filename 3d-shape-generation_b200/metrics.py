@@ -1,5 +1,5 @@
-"""Chamfer core of the reference's metrics.py (:7-47) on the B200 kernels, plus the set-level
-metrics (MMD-CD / COV-CD / 1-NNA-CD) built on the reference's per-pair semantics.
+"""Chamfer core of the reference's metrics.py (:7-47), its Sinkhorn and exact EMD (:49-158) on the B200 kernels, plus the
+set-level metrics (MMD / COV / 1-NNA over CD or EMD) built on the reference's per-pair semantics.
 
 `chamfer_distance(x, y, scaling_factor=1e3)` keeps the reference signature and return type
 (0-dim tensor; batched input -> one scalar averaged over the batch).
@@ -37,6 +37,20 @@ def earth_mover_distance_gpu(x: torch.Tensor, y: torch.Tensor, epsilon: float = 
     return emd.mean() * scaling_factor
 
 
+def earth_mover_distance_exact(x: torch.Tensor, y: torch.Tensor, *, return_assignment: bool = False):
+    """Reference metrics.py:49-92 (`earth_mover_distance_cpu`) on the GPU: an optimal one-to-one matching of the two
+    cube-normalised clouds under Euclidean distance, matched sum divided by 3 (the reference's divisor).  N != M matches
+    min(N, M) pairs.  [N, 3] inputs are promoted to a batch of one; batched input -> the mean over pairs as a 0-dim float32
+    device tensor.  Optimal for distances quantised to 2^-22 (within max(N, M) / 2^22 of the fp64 optimum per pair), at most
+    4096 points per cloud.  return_assignment=True also returns the matched y index of every x, int32 [B, N] (-1: unmatched)."""
+    x = x.unsqueeze(0) if x.dim() == 2 else x
+    y = y.unsqueeze(0) if y.dim() == 2 else y
+    if return_assignment:
+        emd, assign = _lib.emd_exact(x, y, return_assignment=True)
+        return emd.mean(), assign
+    return _lib.emd_exact(x, y).mean()
+
+
 _WARNED = set()
 
 
@@ -65,9 +79,9 @@ def compute_metrics(generated_samples, reference_samples, use_approximate_gpu_em
 
     * Chamfer: the B200 kernels.
     * EMD: `use_approximate_gpu_emd=True` -> the Sinkhorn EMD on the B200 kernels (metrics.py:94-158).  The reference's default is
-      the exact CPU assignment (SciPy Hungarian, metrics.py:49-92), which is out of scope here (SURVEY C8): without an `emd_fn`
-      the default ALSO evaluates the Sinkhorn EMD and says so once -- its values are NOT comparable with the exact EMD (5.995 vs
-      44.307 on the reference's own unit-test inputs).  Pass the reference's `earth_mover_distance_cpu` as `emd_fn` for the exact value.
+      the exact assignment (SciPy Hungarian, metrics.py:49-92).  Without an `emd_fn` the default evaluates the Sinkhorn EMD and
+      says so once -- its values are NOT comparable with the exact EMD (5.995 vs 44.307 on the reference's own unit-test inputs).
+      Pass `emd_fn=pcd_b200.earth_mover_distance_exact` for the exact value on the GPU.
     * recon_loss: binary cross-entropy between the two 32^3 occupancy grids (metrics.py:181), same expression as the reference.
     """
     avg_cd = chamfer_distance(generated_samples, reference_samples)
@@ -75,8 +89,8 @@ def compute_metrics(generated_samples, reference_samples, use_approximate_gpu_em
         avg_emd = emd_fn(generated_samples, reference_samples)
     else:
         if not use_approximate_gpu_emd:
-            _warn_once("emd", "pcd_b200.compute_metrics: the exact CPU EMD (SciPy Hungarian) is not part of the B200 path; returning the "
-                              "Sinkhorn EMD (earth_mover_distance_gpu) instead -- pass emd_fn=<reference earth_mover_distance_cpu> for the exact value")
+            _warn_once("emd", "pcd_b200.compute_metrics: returning the Sinkhorn EMD (earth_mover_distance_gpu), not the reference's "
+                              "default exact EMD -- pass emd_fn=pcd_b200.earth_mover_distance_exact for the exact value")
         avg_emd = earth_mover_distance_gpu(generated_samples, reference_samples)
     if recon_fn is not None:
         recon = recon_fn(generated_samples, reference_samples)
@@ -88,6 +102,30 @@ def compute_metrics(generated_samples, reference_samples, use_approximate_gpu_em
 def chamfer_matrix(G: torch.Tensor, R: torch.Tensor, scaling_factor: float = 1e3) -> torch.Tensor:
     """D[i, j] = chamfer_distance(G[i], R[j])."""
     return _lib.chamfer_matrix(G, R, scaling_factor)
+
+
+_EMD_MATRIX_CHUNK = 4096   # pairs per kernel call: bounds the gathered copies of the clouds (2 x 100 MB at 2048 points)
+
+
+def emd_matrix(G: torch.Tensor, R: torch.Tensor, scaling_factor: float = 1.0) -> torch.Tensor:
+    """D[i, j] = earth_mover_distance_exact(G[i], R[j]) * scaling_factor; every cloud has the same point count.  A set against
+    itself (same tensor) evaluates i <= j only and mirrors it, so emd_matrix(X, X) is symmetric bit for bit."""
+    assert G.shape[1] == R.shape[1], "all clouds must have the same number of points"
+    nG, nR = G.shape[0], R.shape[0]
+    self_mode = G.data_ptr() == R.data_ptr() and G.shape == R.shape and G.stride() == R.stride()
+    if self_mode:
+        ii, jj = torch.triu_indices(nG, nG, device=G.device)
+    else:
+        ii = torch.arange(nG, device=G.device).repeat_interleave(nR)
+        jj = torch.arange(nR, device=G.device).repeat(nG)
+    step = _EMD_MATRIX_CHUNK
+    vals = torch.cat([_lib.emd_exact(G[ii[k:k + step]], R[jj[k:k + step]], scaling_factor)
+                      for k in range(0, ii.numel(), step)]) if ii.numel() else torch.empty(0, device=G.device)
+    out = torch.empty(nG, nR, device=G.device, dtype=torch.float32)
+    out[ii, jj] = vals
+    if self_mode:
+        out[jj, ii] = vals
+    return out
 
 
 def set_metrics_from_matrices(D_gr: torch.Tensor, D_gg: torch.Tensor, D_rr: torch.Tensor) -> dict:
@@ -130,9 +168,13 @@ def _gather_uneven(local: torch.Tensor):
     return torch.cat([p[:c] for p, c in zip(parts, counts)]), sum(counts[:rank])
 
 
-def evaluate_sets(G_local: torch.Tensor, R_local: torch.Tensor, scaling_factor: float = 1e3, *, matrix_fn=None, tile: int = None) -> dict:
+def evaluate_sets(G_local: torch.Tensor, R_local: torch.Tensor, scaling_factor: float = 1e3, *, metric: str = "cd", matrix_fn=None,
+                  tile: int = None) -> dict:
     """MMD-CD / COV-CD / 1-NNA-CD (Achlioptas et al. 2018; Yang et al. 2019 -- not in the reference, SURVEY 0.8) for generated /
     reference clouds sharded over ranks (one process per GPU; shards may be uneven).
+
+    metric="emd" sweeps with `emd_matrix` instead and returns mmd_emd / cov_emd / 1nna_emd with the same definitions, in the
+    reference's EMD unit (`scaling_factor` applies to CD only).  `matrix_fn(A, B, scale)` overrides the matrix function.
 
     One exchange step: NCCL all-gather of both sets.  The three CD matrices are never assembled: they are cut into `tile` x `tile`
     blocks, dealt round-robin to the ranks, and each block is reduced on the spot to row / column minima.  D_gg and D_rr are
@@ -140,7 +182,13 @@ def evaluate_sets(G_local: torch.Tensor, R_local: torch.Tensor, scaling_factor: 
     the sweep costs 2x the G x R pair count (+ n) instead of 3x.  What crosses ranks afterwards is five [n] vectors
     (all_reduce(MIN)), as SURVEY 8(e) sketches.  Ties follow `argmin` on the assembled matrices (first index wins)."""
     import torch.distributed as dist
-    cm = chamfer_matrix if matrix_fn is None else matrix_fn   # injectable so the gloo/CPU test can exercise the exchange
+    if metric not in ("cd", "emd"):
+        raise ValueError("metric must be 'cd' or 'emd'")
+    if metric == "emd":
+        cm, scaling_factor = emd_matrix, 1.0
+    else:
+        cm = chamfer_matrix
+    cm = cm if matrix_fn is None else matrix_fn   # injectable so the gloo/CPU test can exercise the exchange
     multi = dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
     if multi:
         W, rank = dist.get_world_size(), dist.get_rank()
@@ -190,4 +238,4 @@ def evaluate_sets(G_local: torch.Tensor, R_local: torch.Tensor, scaling_factor: 
     # 1-NNA on the concatenation [G | R]: a g row's nearest neighbour is another g unless some r is strictly closer (G columns
     # come first in the assembled matrix, so argmin breaks ties towards G for every row)
     correct = (gg <= gr_row_val).sum() + (rr < gr_col).sum()
-    return {"mmd_cd": float(mmd), "cov_cd": float(cov), "1nna_cd": int(correct) / float(nG + nR)}
+    return {"mmd_" + metric: float(mmd), "cov_" + metric: float(cov), "1nna_" + metric: int(correct) / float(nG + nR)}

@@ -147,6 +147,18 @@ int pcd_chamfer_matrix(const float* G, int32_t nG, const float* R, int32_t nR, i
 int pcd_sinkhorn_emd(const float* x, const float* y, int32_t B, int32_t N, int32_t M, float epsilon, float thresh,
                      int32_t max_iter, float scaling, float* emd, int32_t* iters_out, void* stream);
 
+/* Replaces: metrics.earth_mover_distance_cpu (metrics.py:49-92, SciPy linear_sum_assignment) per pair.  x [B,N,3], y [B,M,3]
+ * device fp32 -> emd[B] (device) = scaling * (sum of |x_i - y_j| over an optimal matching of the cube-normalised clouds) / 3,
+ * the reference's recipe including its divisor of 3 (x_pc.shape[1]).  N != M is allowed: min(N, M) pairs are matched, each
+ * point at most once.  The matching is optimal for the distances quantised to 2^-22, so the value is within n / 2^22 (absolute,
+ * n = max(N, M)) of the fp64 optimum; it is deterministic and does not depend on the other pairs of the batch.
+ * assign_xy [B,N] (device int32, may be NULL) receives the matched y index of every x, or -1 for an unmatched x.  A pair with a
+ * non-finite normalised coordinate (e.g. a cloud whose points are all equal) gets NaN and -1 everywhere.  N, M <= 4096.
+ * The entry synchronises `stream` once, to read back a device flag set when an auction phase exceeds its round cap (then it
+ * returns non-zero; such pairs are NaN). */
+int pcd_emd_exact(const float* x, const float* y, int32_t B, int32_t N, int32_t M, float scaling, float* emd,
+                  int32_t* assign_xy, void* stream);
+
 /* ---- latent-diffusion path (BASELINE config 4) -------------------------------------------------
  * Replaces: LatentDiffusion.__init__/load_state_dict (diffusion.py:361-390) with a
  * SimpleLatentUNetPointNet denoiser (networks.py:962-1106; latent_dim = time_dim = 256, dim = 512)
