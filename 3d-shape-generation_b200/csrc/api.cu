@@ -1080,8 +1080,8 @@ extern "C" int pcd_chamfer_matrix(const float* G, int32_t nG, const float* R, in
 // ------------------------------------------------------------------------------------------
 extern "C" int pcd_sinkhorn_emd(const float* x, const float* y, int32_t B, int32_t N, int32_t M, float epsilon, float thresh,
                                 int32_t max_iter, float scaling, float* emd, int32_t* iters_out, void* stream) {
+    REQ(B > 0 && N > 0 && M > 0, "B, N, M must be positive");   // before the null test: an empty batch has null buffers
     REQ(x && y && emd, "null argument");
-    REQ(B > 0 && N > 0 && M > 0, "B, N, M must be positive");
     REQ(B <= 65535, "at most 65535 pairs per call");
     REQ(epsilon > 0.f && max_iter >= 0, "epsilon must be positive and max_iter non-negative");
     cudaStream_t s = static_cast<cudaStream_t>(stream);

@@ -29,17 +29,18 @@ __global__ void __launch_bounds__(256) cloud_norm_kernel(const float* __restrict
     float4* o = out + static_cast<long long>(blockIdx.x) * N;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     float mn[3] = {3.0e38f, 3.0e38f, 3.0e38f}, mx[3] = {-3.0e38f, -3.0e38f, -3.0e38f};
-    int has_nan = 0;
+    int bad = 0;
     for (int i = tid; i < N; i += 256)
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
             const float v = p[i * 3 + c];
-            has_nan |= (v != v);
+            bad |= !isfinite(v);
             mn[c] = fminf(mn[c], v); mx[c] = fmaxf(mx[c], v);
         }
     // torch.max / torch.min propagate NaN (metrics.py:17-18): ONE NaN coordinate makes the centre, hence every normalised point
-    // and the distance, NaN.  fminf / fmaxf drop NaNs, so the flag is carried separately and poisons the whole cloud below.
-    has_nan = __syncthreads_or(has_nan);
+    // and the distance, NaN.  So does one +-inf coordinate (inf - inf enters the scale).  fminf / fmaxf drop NaNs, so the flag is
+    // carried separately and poisons the whole cloud below.
+    bad = __syncthreads_or(bad);
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
         const float a = warp_min(mn[c]), b = warp_max(mx[c]);
@@ -63,10 +64,15 @@ __global__ void __launch_bounds__(256) cloud_norm_kernel(const float* __restrict
     if (tid == 0) {
         float a = red[0][0];
         for (int w = 1; w < 8; ++w) a = fmaxf(a, red[0][w]);
-        sscale = has_nan ? __int_as_float(0x7fc00000) : a;
+        // Invariant: a cloud whose reference normalisation is not finite comes out NaN in EVERY coordinate of every point, so the
+        // distance kernels need only test element 0's x.  A non-finite input, or a centre that overflows (finite coordinates near
+        // 3e38: max + min is inf), gets a NaN scale here; a degenerate cloud (all points equal, or one point) has scale 0 and
+        // p - c = 0 everywhere, so 0 / 0 below is NaN as in the reference.
+        const bool ok = !bad && isfinite(c0) && isfinite(c1) && isfinite(c2) && isfinite(a);
+        sscale = ok ? a : __int_as_float(0x7fc00000);
     }
     __syncthreads();
-    const float sc = sscale;   // 0 for a degenerate cloud -> NaN, as in the reference
+    const float sc = sscale;
     for (int i = tid; i < N; i += 256)
         o[i] = make_float4(__fdiv_rn(__fsub_rn(p[i * 3], c0), sc), __fdiv_rn(__fsub_rn(p[i * 3 + 1], c1), sc),
                            __fdiv_rn(__fsub_rn(p[i * 3 + 2], c2), sc), 0.f);
@@ -133,8 +139,8 @@ __global__ void __launch_bounds__(128) chamfer_dir_kernel(const float4* __restri
     for (int r = 0; r < R; ++r) {
         const int qi = q0 + r * 128;
         if (qi < Nq) {
-            // a degenerate cloud (all points equal) normalises to 0/0 = NaN everywhere (metrics.py:19-20) and
-            // torch.min / mean propagate it; fminf would silently drop it, so re-inject it here
+            // a degenerate or non-finite cloud normalises to NaN everywhere (metrics.py:19-20, cloud_norm_kernel's invariant)
+            // and torch.min / mean propagate it; fminf would silently drop it, so re-inject it here
             const float qxr = (r & 1) ? qx[r / 2].y : qx[r / 2].x;
             const bool nan_in = (qxr != qxr) || (t[0].x != t[0].x);
             mind[static_cast<long long>(pair) * Nq + qi] = nan_in ? __int_as_float(0x7fc00000) : sqrtf(best[r]);   // L2, not squared (metrics.py:41)

@@ -37,6 +37,7 @@ __global__ void __launch_bounds__(128) emd_cmax_kernel(const float4* __restrict_
     const float4* x = X + static_cast<long long>(pair) * N;
     const float4* y = Y + static_cast<long long>(pair) * M;
     float qx[R], qy[R], qz[R], best[R];
+    int nan_d = 0;
 #pragma unroll
     for (int r = 0; r < R; ++r) {
         const int i = blockIdx.x * (128 * R) + r * 128 + threadIdx.x;
@@ -54,7 +55,9 @@ __global__ void __launch_bounds__(128) emd_cmax_kernel(const float4* __restrict_
 #pragma unroll
             for (int r = 0; r < R; ++r) {
                 const float dx = qx[r] - tv.x, dy = qy[r] - tv.y, dz = qz[r] - tv.z;
-                best[r] = fmaxf(best[r], fmaf(dz, dz, fmaf(dy, dy, dx * dx)));
+                const float d2 = fmaf(dz, dz, fmaf(dy, dy, dx * dx));
+                nan_d |= d2 != d2;
+                best[r] = fmaxf(best[r], d2);
             }
         }
     }
@@ -62,7 +65,10 @@ __global__ void __launch_bounds__(128) emd_cmax_kernel(const float4* __restrict_
 #pragma unroll
     for (int r = 1; r < R; ++r) m = fmaxf(m, best[r]);
     m = block_max_128(m, red);
-    if (threadIdx.x == 0) atomicMax(cmax_bits, __float_as_uint(sqrtf(m)));
+    // torch's C.max() (metrics.py:124) propagates NaN, fmaxf drops it: a NaN distance (a poisoned cloud) makes the batch maximum,
+    // hence every pair's cost, NaN.  Under the unsigned atomicMax the NaN bits 0x7fc00000 beat every finite value and inf.
+    nan_d = __syncthreads_or(nan_d);
+    if (threadIdx.x == 0) atomicMax(cmax_bits, nan_d ? 0x7fc00000u : __float_as_uint(sqrtf(m)));
 }
 
 // One Sinkhorn half-step for the duals of the QUERY cloud:
@@ -126,6 +132,7 @@ __global__ void __launch_bounds__(128) sinkhorn_half_kernel(const float4* __rest
         }
     }
     float err = 0.f;
+    int nan_change = 0;
 #pragma unroll
     for (int r = 0; r < R; ++r) {
         const int i = blockIdx.x * (128 * R) + r * 128 + threadIdx.x;
@@ -133,12 +140,17 @@ __global__ void __launch_bounds__(128) sinkhorn_half_kernel(const float4* __rest
             const float lse = (mx[r] + log2f(sum[r])) * kLn2;
             const float nv = eps * (log_marg - lse);
             float* dst = dual_q + static_cast<long long>(pair) * Nq + i;
-            err = fmaxf(err, fabsf(nv - *dst));
+            const float change = fabsf(nv - *dst);
+            nan_change |= change != change;
+            err = fmaxf(err, change);
             *dst = nv;
         }
     }
     err = block_max_128(err, red);
-    if (threadIdx.x == 0) atomicMax(err_bits, __float_as_uint(err));
+    // torch's max-abs change propagates NaN (a NaN dual, or inf - inf), fmaxf drops it: publish NaN, so that `err < thresh` never
+    // holds and the loop runs max_iter iterations like the reference's (:148-151)
+    nan_change = __syncthreads_or(nan_change);
+    if (threadIdx.x == 0) atomicMax(err_bits, nan_change ? 0x7fc00000u : __float_as_uint(err));
 }
 
 // rowsum[pair][block] = sum over the block's rows i and all j of exp(-lambda*C_ij + alpha_i + beta_j) * C_ij (fixed order)
@@ -174,15 +186,26 @@ __global__ void __launch_bounds__(128) sinkhorn_cost_kernel(const float4* __rest
             st[i] = v;
         }
         __syncthreads();
-#pragma unroll 2
-        for (int j = 0; j < cnt; ++j) {
-            const float4 tv = st[j];
+        // Two-level row sum: 32 targets into `sub`, then `sub` into the row total.  One fp32 accumulator over a whole row rounds
+        // the long tail of small terms away against the large total: the result came out low by ~6e-10 relative per target
+        // (-2.7e-6 at 4100 targets, against fp64).  With 32-target chunks the error stays near 2e-8.
+        for (int j0 = 0; j0 < cnt; j0 += 32) {
+            const int j1 = min(cnt, j0 + 32);
+            float sub[R];
 #pragma unroll
-            for (int r = 0; r < R; ++r) {
-                const float dx = qx[r] - tv.x, dy = qy[r] - tv.y, dz = qz[r] - tv.z;
-                const float c = sqrtf(fmaf(dz, dz, fmaf(dy, dy, dx * dx))) * inv_cmax;
-                acc[r] = fmaf(exp2f(fmaf(c, s2, qa[r] + tv.w)), c, acc[r]);
+            for (int r = 0; r < R; ++r) sub[r] = 0.f;
+#pragma unroll 2
+            for (int j = j0; j < j1; ++j) {
+                const float4 tv = st[j];
+#pragma unroll
+                for (int r = 0; r < R; ++r) {
+                    const float dx = qx[r] - tv.x, dy = qy[r] - tv.y, dz = qz[r] - tv.z;
+                    const float c = sqrtf(fmaf(dz, dz, fmaf(dy, dy, dx * dx))) * inv_cmax;
+                    sub[r] = fmaf(exp2f(fmaf(c, s2, qa[r] + tv.w)), c, sub[r]);
+                }
             }
+#pragma unroll
+            for (int r = 0; r < R; ++r) acc[r] += sub[r];
         }
     }
     float tot = 0.f;

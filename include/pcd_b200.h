@@ -127,13 +127,16 @@ int pcd_linear_bf16(const void* A0, int32_t K0, const void* A1, int32_t K1, cons
 /* Replaces: metrics.chamfer_distance per pair (metrics.py:23-47) incl. normalize_to_cube
  * (metrics.py:7-21).  x [B,N,3], y [B,M,3] device fp32 -> cd[B] (device) =
  * scaling * (mean_i min_j |x_i-y_j| + mean_j min_i |x_i-y_j|) on cube-normalised clouds.
- * idx_xy [B,N] / idx_yx [B,M] (device int32, may be NULL) receive the nearest-neighbour indices. */
+ * idx_xy [B,N] / idx_yx [B,M] (device int32, may be NULL) receive the nearest-neighbour indices.  Like the reference, a pair
+ * with a cloud whose normalisation is not finite (a NaN or +-inf coordinate, a centre that overflows, all points equal or one
+ * point) gets NaN; the other pairs are unaffected. */
 int pcd_chamfer_pairs(const float* x, const float* y, int32_t B, int32_t N, int32_t M, float scaling, float* cd,
                       int32_t* idx_xy, int32_t* idx_yx, void* stream);
 
 /* All-pairs Chamfer matrix out[i*nR + j] = chamfer_distance(G[i], R[j]) (device fp32) for the
  * set metrics MMD-CD / COV / 1-NNA built on the reference's per-pair semantics.  G == R with nG == nR (a set against itself)
- * evaluates the upper triangle only and mirrors it: the values are those of the full sweep (CD is bit-symmetric here). */
+ * evaluates the upper triangle only and mirrors it: the values are those of the full sweep (CD is bit-symmetric here).
+ * An entry with a non-finite normalised cloud is NaN, as in pcd_chamfer_pairs. */
 int pcd_chamfer_matrix(const float* G, int32_t nG, const float* R, int32_t nR, int32_t N, float scaling,
                        float* out, void* stream);
 
@@ -143,7 +146,9 @@ int pcd_chamfer_matrix(const float* G, int32_t nG, const float* R, int32_t nR, i
  * clouds, C = cdist / (ONE maximum over the whole batch), duals from 0, alpha then beta per iteration, stop
  * when both max-abs dual changes over the batch are < thresh or after max_iter iterations.  The cost matrix is
  * never materialised.  Like the reference, the convergence test is a host round trip: this entry synchronises
- * `stream` once per Sinkhorn iteration.  iters_out (host, may be NULL) receives the iteration count. */
+ * `stream` once per Sinkhorn iteration.  iters_out (host, may be NULL) receives the iteration count.  As in the reference, one
+ * pair with a non-finite normalised cloud (see pcd_chamfer_pairs) makes the batch maximum and the convergence test NaN: every
+ * pair of the call is NaN and max_iter iterations run. */
 int pcd_sinkhorn_emd(const float* x, const float* y, int32_t B, int32_t N, int32_t M, float epsilon, float thresh,
                      int32_t max_iter, float scaling, float* emd, int32_t* iters_out, void* stream);
 
@@ -153,7 +158,8 @@ int pcd_sinkhorn_emd(const float* x, const float* y, int32_t B, int32_t N, int32
  * point at most once.  The matching is optimal for the distances quantised to 2^-22, so the value is within n / 2^22 (absolute,
  * n = max(N, M)) of the fp64 optimum; it is deterministic and does not depend on the other pairs of the batch.
  * assign_xy [B,N] (device int32, may be NULL) receives the matched y index of every x, or -1 for an unmatched x.  A pair with a
- * non-finite normalised coordinate (e.g. a cloud whose points are all equal) gets NaN and -1 everywhere.  N, M <= 4096.
+ * non-finite normalised coordinate (see pcd_chamfer_pairs) gets NaN and -1 everywhere; the other pairs are unaffected.
+ * N, M <= 4096.
  * The entry synchronises `stream` once, to read back a device flag set when an auction phase exceeds its round cap (then it
  * returns non-zero; such pairs are NaN). */
 int pcd_emd_exact(const float* x, const float* y, int32_t B, int32_t N, int32_t M, float scaling, float* emd,

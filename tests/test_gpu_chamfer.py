@@ -117,25 +117,32 @@ def test_evaluate_sets_tiled_triangle_schedule_on_the_kernels():
 @pytest.mark.parametrize("n", [1, 2, 7, 33])
 def test_matrix_of_a_set_against_itself_mirrors_the_upper_triangle(n):
     """pcd_chamfer_matrix(G, G) evaluates n (n + 1) / 2 pairs and mirrors them; the values must be those of the full sweep, bit for
-    bit (a clone has another address, so it takes the all-pairs path).  Row 0 of the larger sets is degenerate and one has a NaN."""
+    bit (a clone has another address, so it takes the all-pairs path).  Row 0 of the larger sets is degenerate, one has a NaN and
+    one a +inf in y (inf - inf makes the reference's scale NaN)."""
     g = torch.Generator().manual_seed(100 + n)
     G = torch.randn(n, 300, 3, generator=g).cuda()
     if n >= 7:
         G[0] = 0.25                     # degenerate cloud -> NaN row and column (metrics.py:19-20)
         G[3, 17, 1] = float("nan")
+        G[5, 9, 1] = float("inf")
     full = pcd_b200.chamfer_matrix(G, G.clone())
     tri = pcd_b200.chamfer_matrix(G, G)
     assert tri.shape == (n, n)
+    if n >= 7:
+        bad = torch.zeros(n, dtype=torch.bool, device="cuda")
+        bad[[0, 3, 5]] = True
+        assert torch.equal(torch.isnan(full), bad[:, None] | bad[None, :])
     assert torch.equal(torch.isnan(tri), torch.isnan(full))
     assert torch.equal(torch.nan_to_num(tri, nan=-1.0), torch.nan_to_num(full, nan=-1.0))
     assert torch.equal(torch.nan_to_num(tri, nan=-1.0), torch.nan_to_num(tri.t(), nan=-1.0))
 
 
-@pytest.mark.parametrize("N,M", [(2, 2), (2, 7), (3, 300), (257, 255), (513, 64), (64, 2049), (4500, 4100)])
+@pytest.mark.parametrize("N,M", [(2, 2), (2, 7), (3, 300), (257, 255), (513, 64), (64, 2049), (4500, 4100), (6500, 6400)])
 def test_tiny_and_odd_cloud_sizes_vs_exact_oracle(N, M):
     """Point counts that are no multiple of any tile (the kernels pad with far-away sentinels), down to two points per cloud (one
-    point is degenerate: NaN, tested above) and beyond what the fused kernel's shared memory holds (4500 x 4100 takes the
-    directional passes): values against the exact oracle, indices bit-exact up to ties, all-pairs matrix consistent with the pairs."""
+    point is degenerate: NaN, tested above), up to the fused kernel's shared memory (4500 x 4100 takes 137 of its 200 KB) and
+    beyond it (6500 x 6400 takes the directional passes): values against the exact oracle, indices bit-exact up to ties, all-pairs
+    matrix consistent with the pairs."""
     g = torch.Generator().manual_seed(1000 * N + M)
     x = torch.randn(3, N, 3, generator=g) * torch.rand(3, 1, 3, generator=g)
     y = torch.randn(3, M, 3, generator=g) * torch.rand(3, 1, 3, generator=g) + 0.2
