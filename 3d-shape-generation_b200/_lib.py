@@ -102,6 +102,12 @@ _SIGNATURES = {
     "pcd_vae3d_tap": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
     "pcd_vae3d_profile": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                     C.c_int32, C.POINTER(C.c_int32), C.c_void_p]),
+    "pcd_vae3d_encoder_create": (C.c_int, [C.POINTER(_NamedTensor), C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_void_p)]),
+    "pcd_vae3d_encoder_destroy": (C.c_int, [C.c_void_p]),
+    "pcd_vae3d_encode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
+    "pcd_vae3d_encoder_tap": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
+    "pcd_vae3d_encoder_profile": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.c_void_p]),
     "pcd_voxel_count": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_void_p, C.c_void_p]),
     "pcd_voxel_points": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_void_p, C.c_void_p,
                                    C.c_void_p]),

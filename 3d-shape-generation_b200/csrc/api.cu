@@ -51,15 +51,16 @@ static int get_encode() {
 // 16-bit channels-last grid [nb][D][H][W][C] seen through arbitrary element strides (sw, sh, sd, sb; channel stride 1):
 // box = 64 channels x (bw, bh, bd, bb) voxels, 128B swizzle, zero fill outside the extents (= convolution padding)
 int make_tmap5(CUtensorMap* tm, const void* base, int C, int W, int H, int D, long long nb, long long sw, long long sh,
-               long long sd, long long sb, int bw, int bh, int bd, int bb) {
+               long long sd, long long sb, int bw, int bh, int bd, int bb, int es) {
     if (get_encode()) return 1;
     cuuint64_t gdim[5] = {static_cast<cuuint64_t>(C), static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H),
                           static_cast<cuuint64_t>(D), static_cast<cuuint64_t>(nb)};
     cuuint64_t gstr[4] = {static_cast<cuuint64_t>(sw * 2), static_cast<cuuint64_t>(sh * 2), static_cast<cuuint64_t>(sd * 2),
                           static_cast<cuuint64_t>(sb * 2)};
-    cuuint32_t box[5] = {64u, static_cast<cuuint32_t>(bw), static_cast<cuuint32_t>(bh), static_cast<cuuint32_t>(bd),
+    // es > 1: the box steps es voxels per element along w, h and d (TMA loads boxDim / es elements, so boxDim = count * es)
+    cuuint32_t box[5] = {64u, static_cast<cuuint32_t>(bw * es), static_cast<cuuint32_t>(bh * es), static_cast<cuuint32_t>(bd * es),
                          static_cast<cuuint32_t>(bb)};
-    cuuint32_t estr[5] = {1u, 1u, 1u, 1u, 1u};
+    cuuint32_t estr[5] = {1u, static_cast<cuuint32_t>(es), static_cast<cuuint32_t>(es), static_cast<cuuint32_t>(es), 1u};
     CUresult r = g_encode(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(base), gdim, gstr, box, estr,
                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);

@@ -35,7 +35,7 @@ inline int fail(const std::string& m) { g_pcd_err = m; return 1; }
 #include <cuda.h>
 int make_tmap(CUtensorMap* tm, const void* base, long long rows, long long cols, long long ld, int box_rows);
 int make_tmap5(CUtensorMap* tm, const void* base, int C, int W, int H, int D, long long nb, long long sw, long long sh,
-               long long sd, long long sb, int bw, int bh, int bd, int bb);
+               long long sd, long long sb, int bw, int bh, int bd, int bb, int es = 1);
 
 // Per-handle plan cache.  A plan owns the workspace of one problem shape (GBs at full batch), so only the `cap` most recently
 // used shapes stay resident (PCD_MAX_PLANS, default 4); the least recently used one is destroyed -- after a device

@@ -59,7 +59,7 @@ conv3d_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant
     const int cid = blockIdx.x / CL, num_clusters = gridDim.x / CL;
     const int num_tiles = p.num_m_blocks / CL;
     const int main_stages = p.ngroups * p.cin_kb;
-    const int num_stages = main_stages + (p.res ? p.cin_kb : 0);
+    const int num_stages = main_stages + (p.res ? p.res_kb : 0);
 
     if (warp == 0 && lane == 0) {
         prefetch_tensormap(&tmA0);
@@ -98,7 +98,8 @@ conv3d_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant
                     for (int pl = 0; pl < PL; ++pl) {
                         uint8_t* da = sA + stage * A_STAGE + pl * kCvAPlane;
                         if (is_res) tma_load_5d(da, &tmA1, &full_bar[stage], cb * 64, 0, h0 - p.res_t, d0, b0 + pl * p.batch_plane);
-                        else tma_load_5d(da, &tmA0, &full_bar[stage], cb * 64, p.gdw[g], h0 + p.gdh0[g], d0 + p.gdd[g], b0 + pl * p.batch_plane);
+                        else tma_load_5d(da, &tmA0, &full_bar[stage], cb * 64, p.gdw[g], p.stride * h0 + p.gdh0[g], p.stride * d0 + p.gdd[g],
+                                         b0 + pl * p.batch_plane);
                         for (int t = 0; t < ntap; ++t) {
                             uint8_t* db = sB + stage * B_STAGE + pl * kCvBPlane + t * kCvBTap;
                             if constexpr (CL == 1) {

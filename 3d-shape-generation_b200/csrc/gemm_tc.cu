@@ -231,7 +231,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
                             const int b0 = v0 / (cg.W * cg.H * cg.D) + pl * cg.batch_plane;
                             if (kb < p.kb0) {
                                 const int tap = kb / cg.cin_kb, cb = kb - tap * cg.cin_kb;
-                                tma_load_5d(da, &tmA0, &full_bar[stage], cb * kTileK, w0 + cg.dw[tap], h0 + cg.dh[tap], d0 + cg.dd[tap], b0);
+                                tma_load_5d(da, &tmA0, &full_bar[stage], cb * kTileK, cg.stride * w0 + cg.dw[tap], cg.stride * h0 + cg.dh[tap],
+                                            cg.stride * d0 + cg.dd[tap], b0);
                             } else {
                                 tma_load_5d(da, &tmA1, &full_bar[stage], (kb - p.kb0) * kTileK, w0, h0, d0, b0);
                             }

@@ -129,7 +129,9 @@ struct ConvGeom {
     int W, H, D;                      // input grid
     int batch_plane;                  // lo plane = batch index + batch_plane (5-D tensors keep planes on the batch axis)
     int store5d;                      // 1: the output tile is scattered through a strided 5-D map (transposed conv, one parity class)
-    signed char dw[32], dh[32], dd[32];
+    int stride;                       // 1, or 2 (Conv3d k=4 s=2 p=1): the rows are OUTPUT voxels, tap t reads input voxel
+                                      // stride * o + (dd, dh, dw)[t] through a map that steps 2 input voxels per box element
+    signed char dw[64], dh[64], dd[64];
 };
 
 // Tap-grouped implicit-GEMM 3-D convolution (conv3d_tc.cu): 64 output channels, a 128-voxel tile = bh whole w-lines (bw = W
@@ -142,8 +144,11 @@ struct Conv3dParams {
     int ngroups;                      // (dw, dd) tap groups read through A source 0
     int nt;                           // h-taps per group (1..3)
     int cin_kb;                       // 64-channel blocks per tap
-    int res, res_t;                   // res: append cin_kb shortcut stages from A source 1 (identity weights), read at offset 0 =
-                                      // line res_t of a box loaded at h0 - res_t
+    int res, res_t;                   // res: append res_kb shortcut stages from A source 1 (identity or 1x1 weights), read at
+                                      // offset 0 = line res_t of a box loaded at h0 - res_t
+    int res_kb;                       // 64-channel blocks of the shortcut source
+    int stride;                       // 1, or 2: lines are output lines and the A map steps 2 input voxels per element (h0, d0
+                                      // of a tile are multiplied by 2 before the group offset is added)
     int a_box_bytes;                  // bytes one A load deposits: (bh + nt - 1) * bw * 128
     int batch_plane;                  // lo plane of a grid = batch index + batch_plane
     int b_plane_rows;                 // lo plane of the weights = row + b_plane_rows

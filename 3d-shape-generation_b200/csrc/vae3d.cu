@@ -2,6 +2,7 @@
 // (utils.py:511-539).  The 3-D (transposed) convolutions themselves run on the tcgen05 GEMM of gemm_tc.cu as implicit GEMMs
 // (ConvGeom in pcd_types.h); this file holds what is not a GEMM:
 //   vae3d_final_conv_kernel   decoder.12 (Conv3d 32 -> 1, k = 3, padding 1) + Sigmoid on the channels-last 16-bit grid
+//   vae3d_first_conv_kernel   encoder.0 (Conv3d 1 -> 32, k = 3, padding 1) + ReLU of VAE3DLarge.encode
 //   voxel_count_kernel        per sample: number of voxels above the threshold
 //   voxel_points_kernel       per sample: ordered stream compaction of those voxels into (x, y, z) in [-1, 1]
 #include "pcd_launch.h"
@@ -65,6 +66,66 @@ cudaError_t launch_vae3d_final_conv(const void* x, long long plane_elems, int pl
     const size_t smem = sizeof(float) * (27 * cin + 1);
     if (f16) vae3d_final_conv_kernel<1><<<grid, 256, smem, s>>>(static_cast<const uint16_t*>(x), plane_elems, planes, ldc, cin, D, H, W, nvox_total, w, bias, out);
     else     vae3d_final_conv_kernel<0><<<grid, 256, smem, s>>>(static_cast<const uint16_t*>(x), plane_elems, planes, ldc, cin, D, H, W, nvox_total, w, bias, out);
+    return cudaGetLastError();
+}
+
+// encoder.0 of VAE3DLarge.encode: Conv3d(1 -> 32, k = 3, padding 1) + ReLU on the fp32 occupancy grid [B][32^3], one thread per
+// voxel, written as the dense 32-channel 16-bit rows ([plane][Bpad][32^3][32], hi then rounding-residual plane) that encoder.2
+// reads.  Weights w[27][32] (tap-major) and the bias sit in shared memory.
+template <int F16>
+__global__ void __launch_bounds__(256)
+vae3d_first_conv_kernel(const float* __restrict__ vox, long long nvox_total, const float* __restrict__ w, const float* __restrict__ bias,
+                        uint16_t* __restrict__ hi, uint16_t* __restrict__ lo) {
+    constexpr int G = 32, C = 32;
+    __shared__ float sw[27 * C + C];
+    for (int i = threadIdx.x; i < 27 * C; i += blockDim.x) sw[i] = w[i];
+    if (threadIdx.x < C) sw[27 * C + threadIdx.x] = bias[threadIdx.x];
+    __syncthreads();
+    const long long v = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (v >= nvox_total) return;
+    const int xw = static_cast<int>(v % G), yh = static_cast<int>((v / G) % G), zd = static_cast<int>((v / (G * G)) % G);
+    float acc[C];
+#pragma unroll
+    for (int c = 0; c < C; ++c) acc[c] = sw[27 * C + c];
+    for (int kd = 0; kd < 3; ++kd) {
+        const int z2 = zd + kd - 1;
+        if (z2 < 0 || z2 >= G) continue;
+        for (int kh = 0; kh < 3; ++kh) {
+            const int y2 = yh + kh - 1;
+            if (y2 < 0 || y2 >= G) continue;
+            for (int kw = 0; kw < 3; ++kw) {
+                const int x2 = xw + kw - 1;
+                if (x2 < 0 || x2 >= G) continue;
+                const float x = __ldg(vox + v + ((kd - 1) * G + (kh - 1)) * G + (kw - 1));
+                const float* wt = sw + ((kd * 3 + kh) * 3 + kw) * C;
+#pragma unroll
+                for (int c = 0; c < C; ++c) acc[c] = fmaf(wt[c], x, acc[c]);
+            }
+        }
+    }
+    uint4* ph = reinterpret_cast<uint4*>(hi + v * C);
+    uint4* pl = lo ? reinterpret_cast<uint4*>(lo + v * C) : nullptr;
+#pragma unroll
+    for (int c8 = 0; c8 < C / 8; ++c8) {
+        float f[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) f[j] = fmaxf(acc[c8 * 8 + j], 0.f);
+        const uint32_t h0 = pack16x2(f[0], f[1], F16), h1 = pack16x2(f[2], f[3], F16);
+        const uint32_t h2 = pack16x2(f[4], f[5], F16), h3 = pack16x2(f[6], f[7], F16);
+        ph[c8] = make_uint4(h0, h1, h2, h3);
+        if (pl) {
+            const float2 r0 = unpack16x2(h0, F16), r1 = unpack16x2(h1, F16), r2 = unpack16x2(h2, F16), r3 = unpack16x2(h3, F16);
+            pl[c8] = make_uint4(pack16x2(f[0] - r0.x, f[1] - r0.y, F16), pack16x2(f[2] - r1.x, f[3] - r1.y, F16),
+                                pack16x2(f[4] - r2.x, f[5] - r2.y, F16), pack16x2(f[6] - r3.x, f[7] - r3.y, F16));
+        }
+    }
+}
+
+cudaError_t launch_vae3d_first_conv(const float* vox, long long nvox_total, const float* w, const float* bias, void* hi, void* lo,
+                                    int f16, cudaStream_t s) {
+    const int grid = static_cast<int>((nvox_total + 255) / 256);
+    if (f16) vae3d_first_conv_kernel<1><<<grid, 256, 0, s>>>(vox, nvox_total, w, bias, static_cast<uint16_t*>(hi), static_cast<uint16_t*>(lo));
+    else     vae3d_first_conv_kernel<0><<<grid, 256, 0, s>>>(vox, nvox_total, w, bias, static_cast<uint16_t*>(hi), static_cast<uint16_t*>(lo));
     return cudaGetLastError();
 }
 

@@ -1,9 +1,10 @@
-"""Voxel VAE decoding on the B200 path (SURVEY 8(f) rank 4): the reference's DEFAULT latent-diffusion configuration
+"""Voxel VAE encoding and decoding on the B200 path (SURVEY 8(f) rank 4): the reference's DEFAULT latent-diffusion configuration
 (`LatentDiffusion(vae=VAE3DLarge(...), is_voxel_based=True)`, diffusion.py:362, train_point_ldm.py:161-222).
 
 * `VAE3DLarge` / `ResidualBlock3D` are parameter containers with the reference's exact `state_dict` keys
   (networks.py:471-505, 2208-2264); `decode` (networks.py:2327-2339) runs in the CUDA library (`pcd_vae3d_decode`:
-  implicit-GEMM 3-D convolutions on the tcgen05 kernel).  Encoding and training are out of scope.
+  implicit-GEMM 3-D convolutions on the tcgen05 kernel), and so does `encode` (`pcd_vae3d_encode`: the same kernels plus
+  stride-2 convolutions, learned 1x1 shortcuts, a CUDA-core first layer and fp32 heads).  Training is out of scope.
 * `voxel_tensor_to_point_clouds` (utils.py:511-539) is an ordered stream compaction on the GPU
   (`pcd_voxel_count` + `pcd_voxel_points`), bit-identical to the reference's `torch.where` path.
 """
@@ -38,8 +39,8 @@ class ResidualBlock3D(nn.Module):
 
 class VAE3DLarge(nn.Module):
     """Parameter container mirroring reference networks.py:2208-2264 (same constructor signature, same state_dict keys, so
-    `load_state_dict(strict=True)` works in both directions).  `decode(z)` runs on the B200 kernels; `encode` /
-    `forward` / training are off the sampling path and raise."""
+    `load_state_dict(strict=True)` works in both directions).  `encode(x)`, `decode(z)` and
+    `forward(x)` run on the B200 kernels (inference: eval-mode BatchNorm, no autograd); training is out of scope."""
 
     def __init__(self, input_shape=(32, 32, 32), latent_dim=256, lr=1e-4, kl_warmup_epochs=10, kl_warmup_max_beta=0.1,
                  kl_annealing_epochs=100, *, precision: str = DEFAULT_PRECISION):
@@ -66,6 +67,8 @@ class VAE3DLarge(nn.Module):
             nn.Conv3d(32, 1, kernel_size=3, padding=1), nn.Sigmoid())
         self._engine = None
         self._engine_key = None
+        self._enc_engine = None
+        self._enc_engine_key = None
 
     @classmethod
     def load_from_checkpoint(cls, checkpoint_path, map_location="cpu", **overrides):
@@ -83,11 +86,15 @@ class VAE3DLarge(nn.Module):
     def device(self):
         return self.decoder_input.weight.device
 
-    def engine(self) -> "Vae3dEngine":
+    def _key(self, what):
         dev = self.device
         if dev.type != "cuda":
-            raise _lib.PcdError("VAE3DLarge is on %s: the B200 voxel decoder has no CPU fallback; call .to('cuda')" % dev)
-        key = (dev, self.precision, tuple(p._version for p in self.parameters()), tuple(b._version for b in self.buffers()))
+            raise _lib.PcdError("VAE3DLarge is on %s: the B200 voxel %s has no CPU fallback; call .to('cuda')" % (dev, what))
+        return (dev, self.precision, tuple(p._version for p in self.parameters()), tuple(b._version for b in self.buffers()))
+
+    def engine(self) -> "Vae3dEngine":
+        dev = self.device
+        key = self._key("decoder")
         if self._engine is None or key != self._engine_key:
             if self._engine is not None:
                 self._engine.close()
@@ -100,10 +107,31 @@ class VAE3DLarge(nn.Module):
         """Reference networks.py:2327-2339: z [B, latent] -> voxel probabilities [B, 1, 32, 32, 32] (eval-mode BatchNorm)."""
         return self.engine().decode(z)
 
-    def encode(self, x):
-        raise NotImplementedError("VAE3DLarge.encode is off the sampling path (SURVEY 8: out of scope)")
+    def encoder_engine(self) -> "Vae3dEncoderEngine":
+        key = self._key("encoder")
+        if self._enc_engine is None or key != self._enc_engine_key:
+            if self._enc_engine is not None:
+                self._enc_engine.close()
+            self._enc_engine = Vae3dEncoderEngine(self.state_dict(), self.device, self.precision)
+            self._enc_engine_key = key
+        return self._enc_engine
 
-    forward = encode
+    @torch.no_grad()
+    def encode(self, x: torch.Tensor):
+        """Reference VAE3DLarge.encode: occupancy x [B, 1, 32, 32, 32] -> (mu, logvar), each [B, latent] (eval-mode BatchNorm)."""
+        return self.encoder_engine().encode(x)
+
+    @staticmethod
+    def reparameterize(mu: torch.Tensor, logvar: torch.Tensor) -> torch.Tensor:
+        """mu + eps * std with std = exp(0.5 * logvar) and eps = randn_like(std) (the reference's draw)."""
+        std = torch.exp(0.5 * logvar)
+        return mu + torch.randn_like(std) * std
+
+    @torch.no_grad()
+    def forward(self, x: torch.Tensor):
+        """Reference VAE3DLarge.forward: (decode(reparameterize(mu, logvar)), mu, logvar)."""
+        mu, logvar = self.encode(x)
+        return self.decode(self.reparameterize(mu, logvar)), mu, logvar
 
 
 def is_vae3d_large(vae) -> bool:
@@ -189,6 +217,91 @@ class Vae3dEngine:
         vox = torch.empty(z.shape[0], 1, 32, 32, 32, device=z.device, dtype=torch.float32)
         _lib.check(_lib.lib().pcd_vae3d_profile(self._h, z.data_ptr(), vox.data_ptr(), z.shape[0], ms, fl, names, stride, cap,
                                                 C.byref(n), _lib.stream_ptr(z.device)))
+        return [(names.raw[i * stride:(i + 1) * stride].split(b"\0")[0].decode(), float(ms[i]), float(fl[i])) for i in range(n.value)]
+
+
+class Vae3dEncoderEngine:
+    """Owns the opaque pcd_vae3d_encoder handle built from the encoder half of a VAE3DLarge state_dict (`encoder.*`,
+    `fc_mu.*`, `fc_logvar.*`, with or without the `vae.` prefix)."""
+
+    TAP_SHAPES = {0: (32, 32), 2: (32, 64), 3: (16, 64), 5: (16, 128), 6: (8, 128), 8: (8, 256), 9: (4, 256), 11: (4, 512)}
+
+    def __init__(self, state_dict, device: torch.device, precision: str = DEFAULT_PRECISION):
+        if device.type != "cuda":
+            raise _lib.PcdError("the B200 voxel encoder needs a CUDA device; there is no CPU fallback")
+        if precision not in ("bf16", "bf16x3", "f16", "f16mix"):
+            raise ValueError("precision must be 'bf16', 'bf16x3', 'f16' or 'f16mix' (fp16 hi+lo planes)")
+        items = []
+        for k, v in state_dict.items():
+            k = k[4:] if k.startswith("vae.") else k
+            if k.startswith(("encoder.", "fc_mu.", "fc_logvar.")) and not k.endswith("num_batches_tracked"):
+                items.append(("vae." + k, v))
+        keep, arr = [], (_lib._NamedTensor * max(len(items), 1))()
+        for i, (k, v) in enumerate(items):
+            t = v.detach().to(device="cpu", dtype=torch.float32).contiguous()
+            keep.append(t)
+            arr[i].name, arr[i].data, arr[i].dtype, arr[i].ndim = k.encode(), t.data_ptr(), 0, min(t.dim(), 4)
+            shape = list(t.shape)
+            if len(shape) > 4:      # conv weights are 5-D: fold the kernel axes (pcd_named_tensor carries 4 dims)
+                shape = shape[:3] + [int(torch.tensor(shape[3:]).prod())]
+            for d, n in enumerate(shape):
+                arr[i].shape[d] = n
+        h = C.c_void_p()
+        idx = device.index if device.index is not None else torch.cuda.current_device()
+        _lib.check(_lib.lib().pcd_vae3d_encoder_create(arr, len(items), _lib.PRECISION[precision], idx, C.byref(h)))
+        self._h, self.device, self.precision = h, device, precision
+        self.latent_dim = int(state_dict[[k for k in state_dict if k.endswith("fc_mu.weight")][0]].shape[0])
+
+    def close(self):
+        if getattr(self, "_h", None):
+            _lib.lib().pcd_vae3d_encoder_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @staticmethod
+    def _grid(x: torch.Tensor) -> torch.Tensor:
+        _lib._require_cuda(x, "x")
+        if x.dim() != 5 or tuple(x.shape[1:]) != (1, 32, 32, 32):
+            raise ValueError("x must be [B, 1, 32, 32, 32], got %s" % (tuple(x.shape),))
+        return x.to(torch.float32).contiguous()
+
+    def encode(self, x: torch.Tensor):
+        x = self._grid(x)
+        B = x.shape[0]
+        mu = torch.empty(B, self.latent_dim, device=x.device, dtype=torch.float32)
+        logvar = torch.empty_like(mu)
+        _lib.check(_lib.lib().pcd_vae3d_encode(self._h, x.data_ptr(), mu.data_ptr(), logvar.data_ptr(), B, _lib.stream_ptr(x.device)))
+        return mu, logvar
+
+    def tap(self, x: torch.Tensor, seq_index: int) -> torch.Tensor:
+        """Parity hook: activation after encoder index `seq_index` as [B, C, D, H, W] on the host ([B, 512] for 12)."""
+        x = self._grid(x)
+        B = x.shape[0]
+        if seq_index == 12:
+            out = torch.empty(B, 512, dtype=torch.float32)
+        else:
+            G, Cn = self.TAP_SHAPES.get(seq_index, (1, 1))
+            out = torch.empty(B, G, G, G, Cn, dtype=torch.float32)
+        _lib.check(_lib.lib().pcd_vae3d_encoder_tap(self._h, x.data_ptr(), B, seq_index, out.data_ptr(), out.numel(),
+                                                    _lib.stream_ptr(x.device)))
+        return out if seq_index == 12 else out.permute(0, 4, 1, 2, 3).contiguous()
+
+    def profile(self, x: torch.Tensor):
+        """[(name, ms, algorithmic FLOPs)] of one eager encode, CUDA-event timed per launch."""
+        x = self._grid(x)
+        B = x.shape[0]
+        cap, stride = 64, 48
+        ms, fl = (C.c_float * cap)(), (C.c_double * cap)()
+        names, n = C.create_string_buffer(cap * stride), C.c_int32(0)
+        mu = torch.empty(B, self.latent_dim, device=x.device, dtype=torch.float32)
+        logvar = torch.empty_like(mu)
+        _lib.check(_lib.lib().pcd_vae3d_encoder_profile(self._h, x.data_ptr(), mu.data_ptr(), logvar.data_ptr(), B, ms, fl, names,
+                                                        stride, cap, C.byref(n), _lib.stream_ptr(x.device)))
         return [(names.raw[i * stride:(i + 1) * stride].split(b"\0")[0].decode(), float(ms[i]), float(fl[i])) for i in range(n.value)]
 
 

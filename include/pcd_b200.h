@@ -206,6 +206,25 @@ int pcd_vae3d_tap(pcd_vae3d* h, const float* z, int32_t B, int32_t seq_index, fl
 /* Measurement hook: one eager decode with a CUDA event between launches (same contract as pcd_denoiser_profile). */
 int pcd_vae3d_profile(pcd_vae3d* h, const float* z, float* vox, int32_t B, float* ms_out, double* flops_out, char* names_out,
                       int32_t name_stride, int32_t cap, int32_t* n_out, void* stream);
+/* ---- voxel-VAE encoder ------------------------------------------------------------------------------------------------
+ * Replaces: VAE3DLarge.encode (networks.py, just above decode at :2327): the encoder nn.Sequential of networks.py:2210-2241
+ * (Conv3d 1 -> 32 + ReLU, then ResidualBlock3D(c -> 2c) with a 1x1 `downsample` shortcut and Conv3d(k=4, s=2, p=1) + ReLU per
+ * stage, 32^3 -> 4^3, then Conv3d(512 -> 512, k=4, p=0) + ReLU + Flatten) and fc_mu / fc_logvar (networks.py:2243-2244).
+ * Consumes `vae.encoder.*`, `vae.fc_mu.*` and `vae.fc_logvar.*` (BatchNorm3d folded, eval mode); a missing key is named in
+ * the error.  Its own handle, so decoder-only tables keep working with pcd_vae3d_*.  Precisions as for the decoder. */
+typedef struct pcd_vae3d_encoder pcd_vae3d_encoder;
+int pcd_vae3d_encoder_create(const pcd_named_tensor* tensors, int32_t n_tensors, int32_t precision, int32_t device,
+                             pcd_vae3d_encoder** out);
+int pcd_vae3d_encoder_destroy(pcd_vae3d_encoder* h);
+/* vox [B, 1, 32, 32, 32] device fp32 -> mu, logvar [B, latent] device fp32 */
+int pcd_vae3d_encode(pcd_vae3d_encoder* h, const float* vox, float* mu, float* logvar, int32_t B, void* stream);
+/* Debug/parity tap: run the encoder up to and including nn.Sequential index seq_index (0, 2, 3, 5, 6, 8, 9, 11 or 12 = after
+ * the ReLU, [B][512]) and copy that activation to HOST fp32, channels-last [B][D][H][W][C].  Synchronises. */
+int pcd_vae3d_encoder_tap(pcd_vae3d_encoder* h, const float* vox, int32_t B, int32_t seq_index, float* out_host, int64_t count,
+                          void* stream);
+/* Measurement hook: one eager encode with a CUDA event between launches (same contract as pcd_vae3d_profile). */
+int pcd_vae3d_encoder_profile(pcd_vae3d_encoder* h, const float* vox, float* mu, float* logvar, int32_t B, float* ms_out,
+                              double* flops_out, char* names_out, int32_t name_stride, int32_t cap, int32_t* n_out, void* stream);
 /* Replaces: utils.voxel_tensor_to_point_clouds (utils.py:511-539), called by LatentDiffusion.sample* on the decoded grid
  * (diffusion.py:611-612, 650-651, 704-705).  Two calls because the output is ragged: pcd_voxel_count gives, per sample, the
  * number of voxels with value > threshold; the caller turns the counts into exclusive offsets (int64) and pcd_voxel_points
