@@ -16,7 +16,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("PCD_LIB_PATH") or os.path.join(_HERE, "libpcd_b200.so")   # PCD_LIB_PATH: A/B-compare two builds on one box
 CSRC = os.path.join(_HERE, "csrc")
-SOURCES = ["api.cu", "api_latent.cu", "gemm_tc.cu", "gemm_simt.cu", "chamfer.cu", "emd.cu", "emd_exact.cu", "latent.cu", "latent_mk.cu", "chain_tc.cu", "folding.cu", "api_vae3d.cu", "vae3d.cu", "conv3d_tc.cu"]
+SOURCES = ["api.cu", "api_latent.cu", "gemm_tc.cu", "gemm_simt.cu", "chamfer.cu", "emd.cu", "emd_exact.cu", "latent.cu", "latent_mk.cu", "chain_tc.cu", "folding.cu", "api_vae3d.cu", "vae3d.cu", "conv3d_tc.cu", "api_pointvae.cu"]
 
 PRECISION = {"bf16": 0, "fp32": 1, "bf16x3": 2, "f16": 3, "f16mix": 4}
 SCHED_ROW = 8
@@ -107,6 +107,12 @@ _SIGNATURES = {
     "pcd_vae3d_encode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "pcd_vae3d_encoder_tap": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
     "pcd_vae3d_encoder_profile": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.c_void_p]),
+    "pcd_point_encoder_create": (C.c_int, [C.POINTER(_NamedTensor), C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_void_p)]),
+    "pcd_point_encoder_destroy": (C.c_int, [C.c_void_p]),
+    "pcd_point_encode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
+    "pcd_point_encoder_tap": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
+    "pcd_point_encoder_profile": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
                                             C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.c_void_p]),
     "pcd_voxel_count": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_void_p, C.c_void_p]),
     "pcd_voxel_points": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_void_p, C.c_void_p,

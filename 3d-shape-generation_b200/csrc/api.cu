@@ -99,12 +99,6 @@ int make_tmap(CUtensorMap* tm, const void* base, long long rows, long long cols,
 // ------------------------------------------------------------------------------------------
 // weights
 // ------------------------------------------------------------------------------------------
-struct HostMat {   // folded fp32 layer on the host
-    int cout = 0, k = 0;
-    std::vector<float> w;   // [cout][k]
-    std::vector<float> b;   // [cout]
-};
-
 struct DevLayer {
     int cout = 0, k = 0;
     float* w32 = nullptr;   // [cout][k] fp32
@@ -115,8 +109,8 @@ struct DevLayer {
 
 // conv (k=1) followed by eval-mode BatchNorm1d folded into one affine map (networks.py:46-48):
 //   y = (W x + b - mu) * gamma / sqrt(var + eps) + beta  =  (s*W) x + (s*(b - mu) + beta)
-static bool fold_conv_bn(const TensorTable& tt, const std::string& conv, const std::string& bn, int cout, int cin,
-                         HostMat* out, std::string* err) {
+bool fold_conv_bn(const TensorTable& tt, const std::string& conv, const std::string& bn, int cout, int cin,
+                  HostMat* out, std::string* err) {
     const float *w, *b;
     if (!fetch(tt, conv + ".weight", 1LL * cout * cin, &w, err)) return false;
     if (!fetch(tt, conv + ".bias", cout, &b, err)) return false;
@@ -453,6 +447,31 @@ static int plan_alloc(Plan* pl, void** out, size_t bytes) {
     return 0;
 }
 
+TcShape tc_shape(int epi, int np, long long M, int cout, int K, int num_sms) {
+    TcShape s;
+    if (epi == EPI_MAXPOOL) {
+        s.bn = (np == 1 && M % 256 == 0) ? 256 : 128;
+        s.cl = (cout / 128) % 2 == 0 ? 2 : 1;
+    } else {
+        s.cl = (M / 128) % 2 == 0 ? 2 : 1;
+        // split precision (3 passes, 2 planes): 128-column tiles, or 256-column tiles on the pair MMA where each CTA stages only half
+        // of the B tile (halves the L2->SM bytes per FLOP)
+        const bool wide3 = np == 4 || (np == 3 && s.cl == 2 && cout >= 256 && K >= 512);
+        s.bn = np >= 3 ? (wide3 ? 256 : (cout >= 128 ? 128 : cout)) : (cout >= 256 ? 256 : cout);
+        // live activation bytes under the default order: one row block (128 rows x K x planes read) per CTA.  Measured per layer
+        // (profiles/tile_order_ab_r2.jsonl): n fastest wins where that set is >= 38 MB and the layer has 2..4 weight tiles
+        // (dec4.conv2 in f16mix: 3.68 -> 3.10 ms); with 8 weight tiles (global_feat.0) the default order stays ahead by 1-3 %.
+        const int num_n = cout / s.bn;
+        const double live_mb = static_cast<double>(num_sms) * 128.0 * K * 2.0 * (np >= 3 ? 2 : 1) / (1 << 20);
+        s.tile_order = (num_n >= 2 && num_n <= 4 && live_mb > 30.0) ? 1 : 0;
+    }
+    // pairs run the pair MMA (cta_group::2) on layers with K >= 1024, TMA multicast + per-CTA MMAs elsewhere (measured: +5-6 % on
+    // K >= 1024, -15 % on K <= 512 where per-tile hand-shakes dominate)
+    s.two_sm = (s.cl == 2 && K >= 1024) ? 1 : 0;
+    if (np >= 3 && s.bn == 256) s.two_sm = 1;
+    return s;
+}
+
 static int add_gemm(pcd_denoiser* h, Plan* pl, int layer, const void* a0, int k0, const void* a1, int k1, void* dst,
                     int epi, const float* sample_bias, long long sample_bias_stride) {
     const DevLayer& L = h->L[layer];
@@ -485,11 +504,11 @@ static int add_gemm(pcd_denoiser* h, Plan* pl, int layer, const void* a0, int k0
     p.kb0 = k0 / 64; p.kb1 = k1 / 64;
     p.bias = bias; p.bias_sample_stride = sample_bias_stride; p.rows_per_sample = pl->Npad; p.relu = 1;
     p.gmax = pl->gmax; p.ld_g = 4096; p.n_valid = pl->N; p.num_samples = pl->B; p.call = pl->call;
+    const TcShape sh = tc_shape(epi, op.np, pl->M, L.cout, k0 + k1, h->num_sms);
+    op.bn = sh.bn; op.cl = sh.cl; op.two_sm = sh.two_sm; p.tile_order = sh.tile_order;
     if (epi == EPI_MAXPOOL) {
         // weights take the A role (128 channels per tile), points the B role
-        op.bn = (op.np == 1 && pl->M % 256 == 0) ? 256 : 128;
         p.num_m_blocks = L.cout / 128; p.num_n_blocks = static_cast<int>(pl->M / op.bn);
-        op.cl = p.num_m_blocks % 2 == 0 ? 2 : 1;
         p.a_plane_rows = PLn == 2 ? L.cout : 0; p.b_plane_rows = PLn == 2 ? static_cast<int>(pl->M) : 0; p.out_plane_rows = 0;
         if (make_tmap(&op.a0, L.w16, static_cast<long long>(L.cout) * PLn, L.k, L.k, 128)) return 1;
         op.a1 = op.a0;
@@ -497,11 +516,6 @@ static int add_gemm(pcd_denoiser* h, Plan* pl, int layer, const void* a0, int k0
         op.o = op.a0;
     } else {
         p.num_m_blocks = static_cast<int>(pl->M / 128);
-        op.cl = p.num_m_blocks % 2 == 0 ? 2 : 1;
-        // split precision (3 passes, 2 planes): 128-column tiles, or 256-column tiles on the pair MMA where each CTA stages only half
-        // of the B tile (halves the L2->SM bytes per FLOP)
-        const bool wide3 = op.np == 4 || (op.np == 3 && op.cl == 2 && L.cout >= 256 && k0 + k1 >= 512);
-        op.bn = op.np >= 3 ? (wide3 ? 256 : (L.cout >= 128 ? 128 : L.cout)) : (L.cout >= 256 ? 256 : L.cout);
         p.num_n_blocks = L.cout / op.bn;
         p.out = static_cast<__nv_bfloat16*>(dst); p.ldo = L.cout;
         p.a_plane_rows = PLn == 2 ? static_cast<int>(pl->M) : 0;
@@ -516,17 +530,6 @@ static int add_gemm(pcd_denoiser* h, Plan* pl, int layer, const void* a0, int k0
         if (epi == EPI_STORE) { if (make_tmap_out32(&op.o, dst, Mrows, L.cout, L.cout)) return 1; }
         else op.o = op.a0;
     }
-    if (epi != EPI_MAXPOOL) {
-        // live activation bytes under the default order: one row block (128 rows x K x planes read) per CTA.  Measured per layer
-        // (profiles/tile_order_ab_r2.jsonl): n fastest wins where that set is >= 38 MB and the layer has 2..4 weight tiles
-        // (dec4.conv2 in f16mix: 3.68 -> 3.10 ms); with 8 weight tiles (global_feat.0) the default order stays ahead by 1-3 %.
-        const double live_mb = static_cast<double>(h->num_sms) * 128.0 * (k0 + k1) * 2.0 * (op.np >= 3 ? 2 : 1) / (1 << 20);
-        p.tile_order = (p.num_n_blocks >= 2 && p.num_n_blocks <= 4 && live_mb > 30.0) ? 1 : 0;
-    }
-    // pairs run the pair MMA (cta_group::2) on layers with K >= 1024, TMA multicast + per-CTA MMAs elsewhere (measured: +5-6 % on
-    // K >= 1024, -15 % on K <= 512 where per-tile hand-shakes dominate)
-    op.two_sm = (op.cl == 2 && k0 + k1 >= 1024) ? 1 : 0;
-    if (op.np >= 3 && op.bn == 256) op.two_sm = 1;
     if (np3_one_plane && op.bn != 256) op.out_planes = 2;
     if (layer == L_E3C3) pl->fmtX3 = op.out_planes;
     if (layer == L_E4C3) pl->fmtX4 = op.out_planes;

@@ -37,6 +37,14 @@ int make_tmap(CUtensorMap* tm, const void* base, long long rows, long long cols,
 int make_tmap5(CUtensorMap* tm, const void* base, int C, int W, int H, int D, long long nb, long long sw, long long sh,
                long long sd, long long sb, int bw, int bh, int bd, int bb, int es = 1);
 
+int make_tmap_out32(CUtensorMap* tm, const void* base, long long rows, long long cols, long long ld);
+
+// Tile shape of one tcgen05 GEMM launch (gemm_tc.cu) of a per-point layer: tile columns `bn`, cluster size `cl` (CTA pairs when the
+// A-role blocks pair up), the pair MMA (`two_sm`) and the STORE tile order, from the epilogue, the MMA passes per k-step `np`, the
+// point rows M, the output channels and K.  Shared by every handle that runs per-point layers (defined in api.cu).
+struct TcShape { int bn = 0, cl = 1, two_sm = 0, tile_order = 0; };
+TcShape tc_shape(int epi, int np, long long M, int cout, int K, int num_sms);
+
 // Per-handle plan cache.  A plan owns the workspace of one problem shape (GBs at full batch), so only the `cap` most recently
 // used shapes stay resident (PCD_MAX_PLANS, default 4); the least recently used one is destroyed -- after a device
 // synchronisation, its kernels may still be in flight -- BEFORE the workspace of a new shape is allocated.
@@ -102,3 +110,12 @@ inline bool fetch(const TensorTable& tt, const std::string& name, long long n_ex
     return true;
 }
 
+struct HostMat {   // folded fp32 layer on the host
+    int cout = 0, k = 0;
+    std::vector<float> w;   // [cout][k]
+    std::vector<float> b;   // [cout]
+};
+
+// conv (k=1) followed by eval-mode BatchNorm1d folded into one affine map in double (defined in api.cu); bn empty = bare conv
+bool fold_conv_bn(const TensorTable& tt, const std::string& conv, const std::string& bn, int cout, int cin, HostMat* out,
+                  std::string* err);

@@ -1,6 +1,7 @@
 """Latent-diffusion sampling (reference `LatentDiffusion`, diffusion.py:361-707) on the B200 path:
 `SimpleLatentUNetPointNet` (networks.py:962-1106) as the latent denoiser and
-`SimplePointNetVAE.decode` (networks.py:1144-1154, 1219-1231) as the fused 2048-point decoder.
+`SimplePointNetVAE.decode` (networks.py:1144-1154, 1219-1231) as the fused 2048-point decoder.  `SimplePointNetVAE.encode` /
+`forward` run on the per-point tcgen05 GEMMs with a fused max-pool (`pcd_point_encode`, `PointEncoderEngine`).
 
 Module trees are parameter containers with the reference's exact state_dict keys; forward /
 decode / the loops run in the CUDA library (`pcd_latent_*`).  The reference's default voxel VAE
@@ -59,12 +60,17 @@ class SimpleLatentUNetPointNet(nn.Module):
 
 
 class SimplePointNetVAE(nn.Module):
-    """Parameter container mirroring reference networks.py:1110-1156 (encoder kept only so that
-    state_dicts load strictly; encoding/training are out of scope).  `decode` runs in the library."""
+    """Parameter container mirroring reference networks.py:1110-1156 (same state_dict keys, so `load_state_dict(strict=True)`
+    works in both directions).  `encode(x)`, `decode(z)` and `forward(x)` run in the library (inference: eval-mode BatchNorm,
+    no autograd); training is out of scope.  `precision` selects the encoder's tensor-core precision ('bf16x3', 'f16mix',
+    'bf16' or 'f16'); it is not a hyper-parameter of the reference and does not affect `decode`."""
 
     def __init__(self, num_points, latent_dim=256, hidden_dim=512, lr=1e-4, beta=1e-1, dropout_rate=0.1,
-                 chamfer_lambda=1, voxel_lambda=1, focal_alpha=0.25, focal_gamma=2.00):
+                 chamfer_lambda=1, voxel_lambda=1, focal_alpha=0.25, focal_gamma=2.00, *, precision: str = "bf16x3"):
         super().__init__()
+        self.precision = precision
+        self._enc_engine = None
+        self._enc_engine_key = None
         self.hparams = _HParams(num_points=num_points, latent_dim=latent_dim, hidden_dim=hidden_dim, lr=lr, beta=beta,
                                 dropout_rate=dropout_rate, chamfer_lambda=chamfer_lambda, voxel_lambda=voxel_lambda,
                                 focal_alpha=focal_alpha, focal_gamma=focal_gamma)
@@ -81,9 +87,42 @@ class SimplePointNetVAE(nn.Module):
         """Reference networks.py:1219-1231: latent [B, 256] -> points [B, num_points, 3], on the library's fused decoder."""
         return _own_decoder_engine(self, self.output_layer.out_features // 3).decode(z)
 
+    def encoder_engine(self) -> "PointEncoderEngine":
+        """The encoder handle, rebuilt when the parameters or BatchNorm statistics change."""
+        dev = self.fc_mu.weight.device
+        if dev.type != "cuda":
+            raise _lib.PcdError("SimplePointNetVAE is on %s: the B200 point encoder has no CPU fallback; call .to('cuda')" % dev)
+        key = (dev, self.precision, tuple(p._version for p in self.parameters()), tuple(b._version for b in self.buffers()))
+        if self._enc_engine is None or key != self._enc_engine_key:
+            if self._enc_engine is not None:
+                self._enc_engine.close()
+            self._enc_engine = PointEncoderEngine(self.state_dict(), dev, self.precision)
+            self._enc_engine_key = key
+        return self._enc_engine
+
+    @torch.no_grad()
+    def encode(self, x: torch.Tensor):
+        """Reference SimplePointNetVAE.encode: clouds x [B, N, 3] (any N >= 1) -> (mu, logvar), each [B, latent_dim].
+        BatchNorm runs in eval mode (running statistics) whatever the module's mode.  A cloud with a NaN or infinite coordinate
+        gets NaN in every entry, as in the reference."""
+        return self.encoder_engine().encode(x)
+
+    @staticmethod
+    def reparameterize(mu: torch.Tensor, logvar: torch.Tensor) -> torch.Tensor:
+        """mu + eps * std with std = exp(0.5 * logvar) and eps = randn_like(std) (the reference's draw)."""
+        std = torch.exp(0.5 * logvar)
+        return mu + torch.randn_like(std) * std
+
+    @torch.no_grad()
+    def forward(self, x: torch.Tensor):
+        """Reference SimplePointNetVAE.forward: (decode(reparameterize(mu, logvar)), mu, logvar)."""
+        mu, logvar = self.encode(x)
+        return self.decode(self.reparameterize(mu, logvar)), mu, logvar
+
     @classmethod
     def load_from_checkpoint(cls, checkpoint_path, map_location="cpu", **overrides):
-        """Lightning `.ckpt` dict parsed without Lightning (reference call site train_point_ldm.py:43,190)."""
+        """Lightning `.ckpt` dict parsed without Lightning (reference call site train_point_ldm.py:43,190); `precision=` may be
+        passed as an override."""
         return _vae_from_checkpoint(cls, checkpoint_path, map_location, overrides, strict=True)
 
 
@@ -246,6 +285,90 @@ class LatentEngine:
         out = torch.empty(z.shape[0], self.num_points, 3, device=z.device, dtype=torch.float32)
         _lib.check(_lib.lib().pcd_vae_decode(self._h, z.data_ptr(), out.data_ptr(), z.shape[0], _lib.stream_ptr(z.device)))
         return out
+
+
+class PointEncoderEngine:
+    """Owns the opaque pcd_point_encoder handle built from the encoder half of a SimplePointNetVAE state_dict (`encoder.*`,
+    `fc_mu.*`, `fc_logvar.*`, with or without the `vae.` prefix, so the reference's own module encodes from its `state_dict()`).
+    Only hidden_dim = 512 and latent_dim = 256 (the reference defaults) are supported."""
+
+    def __init__(self, state_dict, device: torch.device, precision: str = "bf16x3"):
+        if device.type != "cuda":
+            raise _lib.PcdError("the B200 point encoder needs a CUDA device; there is no CPU fallback")
+        if precision not in ("bf16", "bf16x3", "f16", "f16mix"):
+            raise ValueError("precision must be 'bf16', 'bf16x3', 'f16' or 'f16mix' (fp16 hi+lo planes)")
+        items = []
+        for k, v in state_dict.items():
+            k = k[4:] if k.startswith("vae.") else k
+            if k.startswith(("encoder.", "fc_mu.", "fc_logvar.")) and not k.endswith("num_batches_tracked"):
+                items.append(("vae." + k, v))
+        keep, arr = [], (_lib._NamedTensor * max(len(items), 1))()
+        for i, (k, v) in enumerate(items):
+            t = v.detach().to(device="cpu", dtype=torch.float32).contiguous()
+            keep.append(t)
+            arr[i].name, arr[i].data, arr[i].dtype, arr[i].ndim = k.encode(), t.data_ptr(), 0, min(t.dim(), 4)
+            for d in range(min(t.dim(), 4)):
+                arr[i].shape[d] = t.shape[d]
+        h = C.c_void_p()
+        idx = device.index if device.index is not None else torch.cuda.current_device()
+        _lib.check(_lib.lib().pcd_point_encoder_create(arr, len(items), _lib.PRECISION[precision], idx, C.byref(h)))
+        self._h, self.device, self.precision = h, device, precision
+        self.latent_dim = 256
+
+    def close(self):
+        if getattr(self, "_h", None):
+            _lib.lib().pcd_point_encoder_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @staticmethod
+    def _clouds(x: torch.Tensor) -> torch.Tensor:
+        if x.dim() != 3 or x.shape[2] != 3:
+            raise ValueError("x must be [B, N, 3], got %s" % (tuple(x.shape),))
+        _lib._require_cuda(x, "x")
+        return x.to(torch.float32).contiguous()
+
+    def encode(self, x: torch.Tensor):
+        """x [B, N, 3] -> (mu, logvar), each [B, 256] fp32 on x's device."""
+        x = self._clouds(x)
+        B, N, _ = x.shape
+        mu = torch.empty(B, self.latent_dim, device=x.device, dtype=torch.float32)
+        logvar = torch.empty_like(mu)
+        _lib.check(_lib.lib().pcd_point_encode(self._h, x.data_ptr(), mu.data_ptr(), logvar.data_ptr(), B, N, _lib.stream_ptr(x.device)))
+        return mu, logvar
+
+    def tap(self, x: torch.Tensor, index: int) -> torch.Tensor:
+        """Parity hook on the host: index 0..11 = the activation after encoder.<index // 3>.conv<index % 3 + 1> (+ BatchNorm +
+        ReLU) as [B, C, N] (the reference's channels-first layout); 12 = the pooled [B, 512]; 13 = encoder.7's output [B, 256]."""
+        x = self._clouds(x)
+        B, N, _ = x.shape
+        if index == 12:
+            out = torch.empty(B, 512, dtype=torch.float32)
+        elif index == 13:
+            out = torch.empty(B, 256, dtype=torch.float32)
+        else:
+            out = torch.empty(B, N, (64, 128, 256, 512)[min(max(index, 0), 11) // 3], dtype=torch.float32)
+        _lib.check(_lib.lib().pcd_point_encoder_tap(self._h, x.data_ptr(), B, N, index, out.data_ptr(), out.numel(),
+                                                    _lib.stream_ptr(x.device)))
+        return out if index >= 12 else out.transpose(1, 2).contiguous()
+
+    def profile(self, x: torch.Tensor):
+        """[(name, ms, useful FLOPs)] of one eager encode, CUDA-event timed per launch group."""
+        x = self._clouds(x)
+        B, N, _ = x.shape
+        cap, stride = 32, 48
+        ms, fl = (C.c_float * cap)(), (C.c_double * cap)()
+        names, n = C.create_string_buffer(cap * stride), C.c_int32(0)
+        mu = torch.empty(B, self.latent_dim, device=x.device, dtype=torch.float32)
+        logvar = torch.empty_like(mu)
+        _lib.check(_lib.lib().pcd_point_encoder_profile(self._h, x.data_ptr(), mu.data_ptr(), logvar.data_ptr(), B, N, ms, fl, names,
+                                                        stride, cap, C.byref(n), _lib.stream_ptr(x.device)))
+        return [(names.raw[i * stride:(i + 1) * stride].split(b"\0")[0].decode(), float(ms[i]), float(fl[i])) for i in range(n.value)]
 
 
 def latent_philox_normal(seed, sample_offset, step, B, D, device):

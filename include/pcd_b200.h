@@ -225,6 +225,27 @@ int pcd_vae3d_encoder_tap(pcd_vae3d_encoder* h, const float* vox, int32_t B, int
 /* Measurement hook: one eager encode with a CUDA event between launches (same contract as pcd_vae3d_profile). */
 int pcd_vae3d_encoder_profile(pcd_vae3d_encoder* h, const float* vox, float* mu, float* logvar, int32_t B, float* ms_out,
                               double* flops_out, char* names_out, int32_t name_stride, int32_t cap, int32_t* n_out, void* stream);
+/* ---- point-VAE encoder -------------------------------------------------------------------------------------------------
+ * Replaces: SimplePointNetVAE.encode (networks.py:1110-1156; encode between __init__ and decode at :1219): four PointNetLayers
+ * (3 -> 64 -> 128 -> 256 -> 512, each three times Conv1d(k=1) + BatchNorm1d + ReLU), AdaptiveMaxPool1d(1) + Flatten,
+ * Linear(512, 256) + ReLU, then fc_mu / fc_logvar.  Consumes `vae.encoder.*`, `vae.fc_mu.*` and `vae.fc_logvar.*` (BatchNorm1d
+ * folded, eval mode); a missing key is named in the error.  Only hidden_dim = 512 and latent_dim = 256 (the reference defaults)
+ * are supported.  Its own handle, so decoder-only tables keep working with pcd_latent_*.  Precisions as for pcd_vae3d. */
+typedef struct pcd_point_encoder pcd_point_encoder;
+int pcd_point_encoder_create(const pcd_named_tensor* tensors, int32_t n_tensors, int32_t precision, int32_t device,
+                             pcd_point_encoder** out);
+int pcd_point_encoder_destroy(pcd_point_encoder* h);
+/* x [B, N, 3] device fp32 (any N >= 1) -> mu, logvar [B, 256] device fp32.  A cloud with a NaN or +-inf coordinate gets NaN in
+ * every mu / logvar entry; the other clouds of the batch do not change. */
+int pcd_point_encode(pcd_point_encoder* h, const float* x, float* mu, float* logvar, int32_t B, int32_t N, void* stream);
+/* Debug/parity tap: run the encoder up to the tapped tensor and copy it to HOST fp32.  index 0..11 = the activation after
+ * encoder.<index / 3>.conv<index % 3 + 1> (+ BatchNorm + ReLU), valid points only, [B][N][C]; 12 = the pooled [B][512];
+ * 13 = encoder.7's output [B][256].  Synchronises. */
+int pcd_point_encoder_tap(pcd_point_encoder* h, const float* x, int32_t B, int32_t N, int32_t index, float* out_host, int64_t count,
+                          void* stream);
+/* Measurement hook: one eager encode with a CUDA event between launches (same contract as pcd_vae3d_encoder_profile). */
+int pcd_point_encoder_profile(pcd_point_encoder* h, const float* x, float* mu, float* logvar, int32_t B, int32_t N, float* ms_out,
+                              double* flops_out, char* names_out, int32_t name_stride, int32_t cap, int32_t* n_out, void* stream);
 /* Replaces: utils.voxel_tensor_to_point_clouds (utils.py:511-539), called by LatentDiffusion.sample* on the decoded grid
  * (diffusion.py:611-612, 650-651, 704-705).  Two calls because the output is ragged: pcd_voxel_count gives, per sample, the
  * number of voxels with value > threshold; the caller turns the counts into exclusive offsets (int64) and pcd_voxel_points
